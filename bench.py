@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — fwd+bwd ms/view of SplatCo's differentiable render hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
 
 A "step" is one training iteration's render work for the `--mv` multi-view batch (BASELINE.json
 configs[1]: Tanks&Temples-shaped, 100k anchors x 10 offsets ~ 1M candidate Gaussians, 980x545, mv=4):
@@ -22,6 +22,11 @@ warp instructions per live pair); `decode_mlp` = the tcgen05 MLP kernels timed w
 oracle rendering; `gpu_baseline` = same-GPU comparators (torch-eager decode, upstream-structure rasterizer);
 `sub_records` = BASELINE configs[2] (C3) at one GPU / configs[3] (C4, one view per GPU) at eight, measured the same way;
 `multi_gpu_check` (N > 1) = one checked step of the view-sharded path on NCCL against a single-process evaluation.
+
+`--dump-outputs DIR` (rank 0): what the last step of the timed loop computed -- every view's rendered image, the summed
+loss and every parameter gradient -- as DIR/<name>.npy in float32, so that two builds can be compared output for
+output (the inputs of the timed steps depend only on the arguments).  Arrays larger than DUMP_MAX_ELEMS are stored as
+the same seeded sample of their entries in every run.
 
 `--impl reference`: the reference's rasterizer is CUDA-only and absent from the mount and its Python
 decode cannot travel to the GPU box (SURVEY.md §0.1, §8c), so this arm times the oracle port of the
@@ -60,6 +65,8 @@ WORKLOADS = {
 }
 SCALE_FACTOR = 0.5       # anchor scale = 0.5 / N^(1/3): projected sigma ~0.5-4 px at these resolutions (SURVEY §8d)
 LEVEL = 2                # activate_level in steady state (train.py:305-307)
+DUMP_MAX_ELEMS = 1 << 19  # --dump-outputs: 2 MB per array; C2 and C3 reach it with 16 arrays (4 images, 12 gradients), ~33 MB
+DUMP_MAX_BYTES = 64 << 20
 
 
 def ncu_evidence():
@@ -181,6 +188,8 @@ class Workload:
         self.copied = [torch.cuda.Event() for _ in range(self.mv)]
         self.info = {}
         self.host_ms = {}
+        self.keep_outputs = False       # --dump-outputs: step() keeps its rendered images and loss in self.last
+        self.last = None
 
     def step(self, host_inputs: bool):
         from splatco_b200.gaussian_renderer import prefilter_voxel, render
@@ -188,8 +197,9 @@ class Workload:
         a, device, mv = self.args, self.device, self.mv
         for p in self.params:
             p.grad = None
+        self.last = None                # (released before this step allocates its own)
         total = None
-        Ms, Vs = [], []
+        Ms, Vs, renders = [], [], []
         if host_inputs:
             self.copy_stream.wait_stream(torch.cuda.current_stream(device))     # the previous step no longer reads the buffers
             with torch.cuda.stream(self.copy_stream):
@@ -208,11 +218,29 @@ class Workload:
             loss = l1_ssim_loss(pkg["render"], gt, 0.2) + 0.01 * (pkg["scaling"].prod(dim=1).mean() if a.torch_scaling_reg else scaling_reg(pkg["scaling"]))
             total = loss if total is None else total + loss
             Ms.append(pkg["radii"].shape[0]); Vs.append(pkg["selection_mask"].shape[0] // self.cfg["K"])
+            if self.keep_outputs:
+                renders.append(pkg["render"].detach())
         total.backward()
         if self.bucket is not None:
             self.bucket.allreduce()
+        if self.keep_outputs:
+            self.last = (renders, total.detach())
         self.info["M"], self.info["V"] = float(np.mean(Ms)), float(np.mean(Vs))
         return float(total.item()) if host_inputs else total
+
+    def outputs(self):
+        """Host copies (dump_sample) of what the last step() handed its caller: the rendered image of every view, the
+        summed loss and the gradient of every parameter (None gradients left out), keyed by the names --dump-outputs
+        writes."""
+        renders, loss = self.last
+        out = {f"render_view{v}": r for v, r in enumerate(renders)}
+        out["loss"] = loss
+        pc = self.pc
+        named = {k: getattr(pc, k) for k in ("_anchor", "_offset", "_anchor_feat", "_scaling")}
+        for m in ("mlp_opacity", "mlp_cov", "mlp_color", "feat_planes"):
+            named.update({f"{m}.{k}": p for k, p in getattr(pc, m).named_parameters()})
+        out.update({f"grad.{k}": p.grad for k, p in named.items() if p.grad is not None})
+        return {k: dump_sample(t.cpu().numpy()) for k, t in out.items()}
 
     def timed(self, fn, n, host_inputs, tag=None):
         import torch.distributed as dist
@@ -300,6 +328,27 @@ class Workload:
         return float(np.mean(Rs)), float(np.mean(visited or [0])), float(np.mean(live or [0]))
 
 
+def dump_sample(a):
+    """`a` as float32; an array of more than DUMP_MAX_ELEMS entries becomes its entries at DUMP_MAX_ELEMS positions
+    drawn (seed 0, sorted) from its flattened shape, the same positions in every run."""
+    a = np.asarray(a, np.float32)
+    if a.size > DUMP_MAX_ELEMS:
+        idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+        a = a.reshape(-1)[idx]
+    return a
+
+
+def dump_outputs(d, arrays):
+    """Writes d/<name>.npy (float32) for every array, or nothing if they add up to more than DUMP_MAX_BYTES."""
+    arrays = {k: np.asarray(a, np.float32) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total / 2**20:.1f} MB is more than {DUMP_MAX_BYTES >> 20} MB")
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 def stage_table(w: Workload, stage_sum, ms_stage, R, M, V):
     cfg = w.cfg
     N, H, W = cfg["N"], cfg["H"], cfg["W"]
@@ -348,9 +397,11 @@ def warm_until_quiescent(w, device, world, limit=24, batch=4):
     return extra
 
 
-def sub_record(args, name, device, rank, world, steps=4, warm=3):
-    """A short measurement of another BASELINE config inside the same bench line: value, e2e, dominant-stage roofline."""
+def sub_record(args, name, device, rank, world, warm=3):
+    """A measurement of another BASELINE config inside the same bench line (--steps timed steps): value, e2e,
+    dominant-stage roofline."""
     from splatco_b200 import profiling
+    steps = args.steps
     w = Workload(args, name, device, rank, world)
     for _ in range(warm):
         w.step(False)
@@ -585,7 +636,7 @@ def multi_gpu_check(w: Workload):
 
 def run_ours(args):
     import torch.distributed as dist
-    from splatco_b200 import _lib, profiling
+    from splatco_b200 import _lib, decode, profiling
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -596,6 +647,7 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=device)
     L = _lib.lib()
     w = Workload(args, args.workload, device, rank, world)
+    w.keep_outputs = bool(args.dump_outputs) and rank == 0
     cfg, mv = w.cfg, w.mv
     H, W = cfg["H"], cfg["W"]
     # the GPU side of the `parity` block: view 0 at Q0 = 0 BEFORE anything updates the parameters (compared with the
@@ -617,9 +669,16 @@ def run_ours(args):
     # peer access is enabled (multi-GPU), and the pool keeps growing by a block every few steps for a while (how many
     # buffers of a size are alive at once depends on how far the host runs ahead)
     warm_extra = warm_until_quiescent(w, device, world)
+    # the training-time plane-feature noise of a decode call is seeded from torch's seed and a per-process call counter:
+    # fixing both here makes the timed steps' inputs depend on the arguments only, not on the process or on how many
+    # warm-up steps the allocator needed
+    torch.manual_seed(0)
+    decode._noise_calls = 0
     launches0 = L.splatco_launch_count()
     ms_dev = w.timed(w.step, args.steps, False)
     launches = L.splatco_launch_count() - launches0
+    dumped = w.outputs() if w.keep_outputs else None
+    w.keep_outputs, w.last = False, None
     ms_e2e = w.timed(w.step, args.steps, True)
     clocks = sampler.stop() if rank == 0 else None
     # per-stage CUDA-event times come from a separate pass (two event records per stage would otherwise
@@ -750,6 +809,8 @@ def run_ours(args):
             base, parity = cpu_baseline(cfg, parity_gpu)
             out["cpu_baseline"] = base
             out["parity"] = parity
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -918,7 +979,13 @@ def main():
                          "0 = the first 12 000 iterations (train.py:305-307, SURVEY §8d times both)")
     ap.add_argument("--torch-scaling-reg", action="store_true",
                     help="scaling regulariser with torch ops as train.py:195 writes it (its prod backward syncs with the host every view)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's images, loss and parameter gradients to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed (--impl ours)")
     global LEVEL
     LEVEL = args.level
     if args.impl == "reference":

@@ -29,6 +29,30 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert p.returncode == 0 and p.stdout.strip() == ""
 
 
+def test_dump_outputs_samples_large_arrays_at_fixed_positions(tmp_path):
+    """--dump-outputs: small arrays are written whole, a large one as the same seeded sample in every call, all float32;
+    a dump over the size limit writes no file."""
+    import numpy as np
+    import pytest
+    sys.path.insert(0, ROOT)
+    import bench
+    big = np.arange(3 * bench.DUMP_MAX_ELEMS, dtype=np.float32).reshape(3, -1)
+    arrays = {"loss": np.array(2.5, np.float32), "grad.small": np.ones((4, 3), np.float64), "render_view0": big}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {k: bench.dump_sample(v) for k, v in arrays.items()})
+    too_big = {f"render_view{v}": big for v in range(bench.DUMP_MAX_BYTES // big.nbytes + 1)}
+    with pytest.raises(RuntimeError):
+        bench.dump_outputs(str(tmp_path / "c"), too_big)
+    assert not (tmp_path / "c").exists()
+    a = {f: np.load(str(tmp_path / "a" / f)) for f in os.listdir(str(tmp_path / "a"))}
+    assert sorted(a) == ["grad.small.npy", "loss.npy", "render_view0.npy"]
+    assert all(v.dtype == np.float32 for v in a.values())
+    assert a["loss.npy"].shape == () and a["grad.small.npy"].shape == (4, 3)
+    s = a["render_view0.npy"]
+    assert s.shape == (bench.DUMP_MAX_ELEMS,) and np.all(np.diff(s) > 0) and np.isin(s, big).all()
+    assert np.array_equal(s, np.load(str(tmp_path / "b" / "render_view0.npy")))
+
+
 def test_committed_evidence_is_readable_by_the_bench():
     """The roofline object takes `traffic` and the issue-slot numbers from the newest committed ncu capture and `peak` from
     MEASURED_PEAKS.json: both helpers must parse what is in the tree (a malformed file would only show up on the GPU box)."""

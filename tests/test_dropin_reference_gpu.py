@@ -34,7 +34,8 @@ REF = os.path.join(ROOT, "oracle", "_ref")
 
 def _reference_modules():
     if not os.path.exists(os.path.join(REF, "scene", "gaussian_model.py")):
-        pytest.skip("oracle/_ref is not staged (python oracle/build_ref.py needs /root/reference)")
+        pytest.skip("needs the original SplatCo Python sources staged under oracle/_ref by oracle/build_ref.py; the "
+                    "repository does not include them (its decode is pinned by tests/golden/decode_*.npz)")
     import splatco_shims
     splatco_shims.install(hot_path="rasterizer")          # option A aliasing; the reference's gaussian_renderer stays its own
     if REF not in sys.path:
