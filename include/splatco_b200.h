@@ -145,7 +145,7 @@ int splatco_blend_bwd_upstream(int P, int64_t R, int H, int W, const float *bg, 
 /* A/B switch of the blend kernels (process-wide; timing and debugging only; 0 keeps the current choice).
  *   fwd: 1 = warp-synchronous walk of the patch masks (one splat per warp step), 2 = per-pixel candidate lists from
  *        per-row alpha >= 1/255 spans, every lane walks its own list (default)
- *   bwd: 1 = per-visit nine-sum transposition buffer, 2 = two-value matrix-form reduction on mma.sync (default),
+ *   bwd: 1 = per-visit nine-sum transposition buffer, 2 = two-value matrix-form reduction with constant-weight FMAs (default),
  *        3 = the same with 256-splat batches
  * Environment: SPLATCO_BLEND_FWD, SPLATCO_BLEND_BWD. */
 int splatco_blend_set_impl(int fwd, int bwd);

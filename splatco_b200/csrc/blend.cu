@@ -54,6 +54,17 @@ __device__ __forceinline__ float eval_p2(const float4 &k0, float c2, float u, fl
     return fmaf(c2 * dy, dy, t * dx);
 }
 
+// Both cull filters (the bounding box below, the row spans of splat_patch_words) solve the conic's quadratic from
+// det = a2 c2 - b2^2 / 4.  For needle-shaped splats that is a cancellation: its relative error, and that of the pair
+// test's own p2 evaluation, is about eps * a2 c2 / det, which outgrows the fixed margins of the solutions (0.2 % of
+// tau2, 0.02 px) -- on needles of screen sigma 1000 px and more the row spans dropped pairs the per-pixel test
+// accepts, far out on the needle's flank (tests/test_blend_filters_gpu.py).  Above det / (a2 c2) = 2^-10 the error is
+// about 6e-5, 30x inside the margin; conics worse than that are not culled.
+constexpr float kMinDetRatio = 1.0f / 1024.0f;
+__device__ __forceinline__ bool conic_cullable(float a2, float c2, float det) {
+    return det > 0.f && det > kMinDetRatio * (a2 * c2);
+}
+
 // sx, sy: splat centre relative to the tile centre.  Returns the log2-domain coefficients and the
 // 8-bit patch mask (bit w = warp w's 8x4 patch may see alpha >= 1/255).
 __device__ __forceinline__ SplatCoef splat_setup(float sx, float sy, float A, float B, float C, float op, float r,
@@ -67,7 +78,7 @@ __device__ __forceinline__ SplatCoef splat_setup(float sx, float sy, float A, fl
     const float tau2 = lo - kLog2Inv255;
     uint32_t m = 0;
     const float det = a2 * c2 - 0.25f * b2 * b2;        // > 0 for a valid conic
-    if (tau2 > 0.f && det > 0.f) {
+    if (tau2 > 0.f && conic_cullable(a2, c2, det)) {
         const float t = tau2 * 1.002f + 1e-3f;
         const float inv = t / det;
         const float ex = sqrtf(fmaxf(-c2 * inv, 0.f)) + 0.02f;
@@ -80,7 +91,7 @@ __device__ __forceinline__ SplatCoef splat_setup(float sx, float sy, float A, fl
 #pragma unroll
         for (int w = 0; w < 8; ++w) m |= (((xb >> (w & 1)) & 1u) & ((yb >> (w >> 1)) & 1u)) << w;
     } else if (tau2 > 0.f) {
-        m = 0xffu;                                      // degenerate conic: never cull
+        m = 0xffu;                                      // degenerate or ill-conditioned conic: never cull
     }
     s.mask8 = m;
     return s;
@@ -220,7 +231,7 @@ __device__ __forceinline__ void splat_patch_words(float sx, float sy, float a2, 
         for (int w = 0; w < 8; ++w) pm[w] = 0;
         return;
     }
-    if (det > 0.f && a2 < 0.f) {
+    if (conic_cullable(a2, c2, det) && a2 < 0.f) {
         const float t = tau2 * 1.002f + 1e-3f;
         const float inv_a = rcp_approx(-a2);             // 1 / alpha, alpha = -a2 > 0
         const float at = -a2 * t;
@@ -238,7 +249,7 @@ __device__ __forceinline__ void splat_patch_words(float sx, float sy, float a2, 
         }
     } else {
 #pragma unroll
-        for (int w = 0; w < 8; ++w) rows2[w] = 0xffffffffu;       // degenerate conic: never cull
+        for (int w = 0; w < 8; ++w) rows2[w] = 0xffffffffu;       // degenerate or ill-conditioned conic: never cull
     }
 #pragma unroll
     for (int yq = 0; yq < 4; ++yq) {                    // rows 4yq..4yq+3: low bytes -> left patch, high bytes -> right patch
