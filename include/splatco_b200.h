@@ -160,6 +160,34 @@ int splatco_preprocess_bwd(int P, const float *means3D, const float *scales, int
                            const float *dL_dmean2D, const float *dL_dconic, float *dL_dmeans3D,
                            float *dL_dscales, float *dL_drots, void *stream);
 
+/* ---- depth and alpha maps (opt-in; the colour-only entry points above are unchanged) ----------
+ * Same walk and contributor set as the colour: for each pixel
+ *   depth[p] = sum_i z_i alpha_i T_i   (view-space z of each Gaussian, background 0: ACCUMULATED depth;
+ *                                       the expected depth is depth / alpha, which the caller forms)
+ *   alpha[p] = 1 - T_final[p]
+ * These entry points always run the v2 blend kernels; splatco_blend_set_impl does not apply to them.
+ *
+ * blend_fwd_depth_alpha: what splatco_blend_fwd computes (out_color, and final_T / n_contrib in the image workspace,
+ * bit for bit), plus the caller-owned maps out_depth[H,W] and out_alpha[H,W]. */
+int splatco_blend_fwd_depth_alpha(int64_t R, int H, int W, const float *bg, const void *geom, const void *binning,
+                                  void *image, float *out_color /* [3,H,W] */, float *out_depth /* [H,W] */,
+                                  float *out_alpha /* [H,W] */, void *stream);
+/* blend_bwd_depth_alpha: the backward of the three maps.  Any of dL_dpix [3,H,W], dL_ddepth_map [H,W] and
+ * dL_dalpha_map [H,W] may be NULL (= zero), but not all three.  Like splatco_blend_bwd it ACCUMULATES into
+ * caller-zeroed dL_dmean2D, dL_dconic, dL_dopacity, dL_dcolor, and into dL_ddepth[P] (dL / d view-space z), which
+ * splatco_preprocess_bwd_depth takes on to dL_dmeans3D. */
+int splatco_blend_bwd_depth_alpha(int P, int64_t R, int H, int W, const float *bg, const void *geom,
+                                  const void *binning, const void *image, const float *dL_dpix,
+                                  const float *dL_ddepth_map, const float *dL_dalpha_map, float *dL_dmean2D,
+                                  float *dL_dconic, float *dL_dopacity, float *dL_dcolor, float *dL_ddepth,
+                                  void *stream);
+/* preprocess_bwd_depth: splatco_preprocess_bwd plus dL_ddepth[P] . (dz_view / dmean3D) in dL_dmeans3D. */
+int splatco_preprocess_bwd_depth(int P, const float *means3D, const float *scales, int scale_stride,
+                                 const float *rots, float scale_mod, const float *view, const float *proj,
+                                 float tanfovx, float tanfovy, int H, int W, const int32_t *radii,
+                                 const float *dL_dmean2D, const float *dL_dconic, float *dL_dmeans3D,
+                                 float *dL_dscales, float *dL_drots, const float *dL_ddepth, void *stream);
+
 /* ---- anchor decode: replaces generate_neural_gaussians -----------------------------------------
  * (gaussian_renderer/__init__.py:18-116; FeaturePlanes.forward scene/gaussian_model.py:149-169;
  * PlaneGrid scene/grids.py:146-201; heads scene/gaussian_model.py:316-337).

@@ -46,6 +46,9 @@ SIGNATURES = {
     "splatco_blend_bwd_upstream": (_i, [_i, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "splatco_blend_census": (_i, [_i64, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "splatco_preprocess_bwd": (_i, [_i, _vp, _vp, _i, _vp, _f, _vp, _vp, _f, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "splatco_blend_fwd_depth_alpha": (_i, [_i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "splatco_blend_bwd_depth_alpha": (_i, [_i, _i64, _i, _i] + [_vp] * 13),
+    "splatco_preprocess_bwd_depth": (_i, [_i, _vp, _vp, _i, _vp, _f, _vp, _vp, _f, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     # decode: descriptor / gradient structs are passed with ctypes.byref (see decode.py)
     "splatco_pack_planes": (_i, [_i, _i] + [_vp] * 7),
     "splatco_unpack_planes_add": (_i, [_i, _i] + [_vp] * 7),

@@ -20,6 +20,7 @@
 //           with constant weights).  The defaults; see the comments at the kernels.
 #include "common.cuh"
 #include <stdlib.h>
+#include <type_traits>
 
 namespace splatco {
 
@@ -258,14 +259,22 @@ __device__ __forceinline__ void splat_patch_words(float sx, float sy, float a2, 
     }
 }
 
+//
+// DA (depth / alpha maps): the view-space depth z of each staged splat rides next to its blue channel (one float2 load
+// per live pair instead of one float), D = sum z alpha T is accumulated like a fourth colour channel with background 0,
+// and the kernel also writes depth[pid] = D and alpha[pid] = 1 - T.  Same walk, same decisions: colour, final_T and
+// n_contrib are those of blend_fwd2_kernel<false>.
+template <bool DA>
 __global__ void __launch_bounds__(BLEND_THREADS, 5)
 blend_fwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ point_list,
                   const float4 *__restrict__ rec, int W, int H, int gx, const float *__restrict__ bg,
                   float *__restrict__ out_color, float *__restrict__ final_T,
-                  int32_t *__restrict__ n_contrib, const uint32_t *__restrict__ order) {
+                  int32_t *__restrict__ n_contrib, const uint32_t *__restrict__ order,
+                  float *__restrict__ out_depth = nullptr, float *__restrict__ out_alpha = nullptr) {
+    using BZ = std::conditional_t<DA, float2, float>;           // blue (and z)
     __shared__ float4 s_k0[BLEND_BATCH];
     __shared__ float4 s_k1[BLEND_BATCH];
-    __shared__ float s_b[BLEND_BATCH];
+    __shared__ BZ s_b[BLEND_BATCH];
     __shared__ uint32_t s_cand[BLEND_WORDS][BLEND_THREADS];      // [32-splat word][pixel thread]
     const int tile = order ? (int)order[blockIdx.x] : (int)blockIdx.x;
     const int tile_x = tile % gx, tile_y = tile / gx;
@@ -277,7 +286,7 @@ blend_fwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
     const float cx = (float)(tile_x * TILE) + 7.5f, cy = (float)(tile_y * TILE) + 7.5f;
     int todo = range.y - range.x;
     bool done = !inside;
-    float T = 1.0f, C0 = 0.f, C1 = 0.f, C2 = 0.f;
+    float T = 1.0f, C0 = 0.f, C1 = 0.f, C2 = 0.f, D = 0.f;
     int last_contributor = 0;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
@@ -295,7 +304,8 @@ blend_fwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
                 const float sx = r0.x - cx, sy = r0.y - cy;
                 const float a2 = -0.5f * kLog2e * r0.z, c2 = -0.5f * kLog2e * r1.x, b2 = -kLog2e * r0.w;
                 const float lo = r1.y > 0.f ? __log2f(r1.y) : -1e30f;
-                s_k0[j] = make_float4(sx, sy, a2, b2); s_k1[j] = make_float4(c2, lo, r1.z, r1.w); s_b[j] = r2.x;
+                s_k0[j] = make_float4(sx, sy, a2, b2); s_k1[j] = make_float4(c2, lo, r1.z, r1.w);
+                if constexpr (DA) s_b[j] = make_float2(r2.x, r2.y); else s_b[j] = r2.x;
                 splat_patch_words(sx, sy, a2, b2, c2, lo, pm);
             }
 #pragma unroll
@@ -330,7 +340,13 @@ blend_fwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
                     const float test_T = T * (1.0f - alpha);
                     if (test_T < 0.0001f) { done = true; break; }
                     const float wgt = alpha * T;
-                    C0 = fmaf(k1.z, wgt, C0); C1 = fmaf(k1.w, wgt, C1); C2 = fmaf(s_b[j], wgt, C2);
+                    if constexpr (DA) {
+                        const float2 bz = s_b[j];
+                        C0 = fmaf(k1.z, wgt, C0); C1 = fmaf(k1.w, wgt, C1); C2 = fmaf(bz.x, wgt, C2);
+                        D = fmaf(bz.y, wgt, D);
+                    } else {
+                        C0 = fmaf(k1.z, wgt, C0); C1 = fmaf(k1.w, wgt, C1); C2 = fmaf(s_b[j], wgt, C2);
+                    }
                     T = test_T;
                     last_contributor = pos0 + j;
                 }
@@ -344,6 +360,10 @@ blend_fwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
         out_color[pid] = C0 + T * bg[0];
         out_color[HW + pid] = C1 + T * bg[1];
         out_color[2 * HW + pid] = C2 + T * bg[2];
+        if constexpr (DA) {
+            out_depth[pid] = D;
+            out_alpha[pid] = 1.0f - T;
+        }
     }
 }
 
@@ -537,22 +557,34 @@ blend_bwd_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ p
 // epilogue turns the raw pixel moments into the moments about the splat centre (S_x = sx S - S_u, ...) and issues the
 // global REDs, once per (warp, splat) like before.  (An mma.sync variant of this flush -- 2xTF32 / 3xTF32 -- was
 // measured 13 % slower than the transposition-buffer kernel: the legacy tensor path is slow on sm_100a.)
+//
+// DA (depth / alpha maps): depth is a fourth colour channel with background 0 and alpha = 1 - T_final.  The staged
+// record carries z in its free slot [2].w; the lane keeps one more suffix recurrence (ar3 / lc3) and adds
+// (z - ar3) T g_D to dL/dalpha; the alpha map's gradient g_A enters through the per-pixel constant:
+// d(1 - T_final)/dalpha_i = T_final / (1 - alpha_i), so neg_Tf_bg = -T_final (bg . dL/dpix - g_A).  dL/dz of a splat is
+// sum_pixels alpha T g_D: one more constant-weight dot product of the parked alpha T column against a fourth row
+// (g_D) of the patch's dL/dpixel table, issued by the fh == 0 half of the flush.
 constexpr int MR_ROWS = 16, MR_STRIDE = 36;
 constexpr int MR_WARP_FLOATS = 2 * MR_ROWS * MR_STRIDE + 3 * 32 + MR_ROWS;     // X_g, X_d, dL/dpixel table, slot of each row
-template <int BATCH> constexpr size_t bwd2_smem() { return (size_t)BATCH * 48 + (size_t)(BLEND_THREADS / 32) * MR_WARP_FLOATS * sizeof(float); }
+template <bool DA> constexpr int kMrWarpFloats = DA ? MR_WARP_FLOATS + 32 : MR_WARP_FLOATS;   // + g_D row
+template <int BATCH, bool DA = false> constexpr size_t bwd2_smem() {
+    return (size_t)BATCH * 48 + (size_t)(BLEND_THREADS / 32) * kMrWarpFloats<DA> * sizeof(float);
+}
 
-template <int BATCH>
+template <int BATCH, bool DA>
 __global__ void __launch_bounds__(BLEND_THREADS, BATCH == 256 ? 4 : 3)
 blend_bwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ point_list,
                   const float4 *__restrict__ rec, int W, int H, int gx, const float *__restrict__ bg,
                   const float *__restrict__ final_T, const int32_t *__restrict__ n_contrib,
                   const float *__restrict__ dL_dpix, float *__restrict__ dL_dmean2D,
                   float *__restrict__ dL_dconic, float *__restrict__ dL_dopacity,
-                  float *__restrict__ dL_dcolor, const uint32_t *__restrict__ order) {
+                  float *__restrict__ dL_dcolor, const uint32_t *__restrict__ order,
+                  const float *__restrict__ dL_ddmap = nullptr, const float *__restrict__ dL_damap = nullptr,
+                  float *__restrict__ dL_ddepth = nullptr) {
     constexpr int WORDS = BATCH / 32, PER_THREAD = BATCH / BLEND_THREADS;
     extern __shared__ float4 s_dyn4[];
     float4 *const s_rec = s_dyn4;                                                   // [BATCH * 3]
-    float *const s_buf_all = reinterpret_cast<float *>(s_dyn4 + BATCH * 3);         // [8][MR_WARP_FLOATS]
+    float *const s_buf_all = reinterpret_cast<float *>(s_dyn4 + BATCH * 3);         // [8][kMrWarpFloats<DA>]
     __shared__ uint32_t s_mask[8][WORDS];
     __shared__ int s_max[BLEND_THREADS / 32];
     const int tile = order ? (int)order[blockIdx.x] : (int)blockIdx.x;
@@ -568,16 +600,30 @@ blend_bwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
     const int last = inside ? n_contrib[pid] : 0;
     float T = T_final;
     float dp0 = 0.f, dp1 = 0.f, dp2 = 0.f;
-    if (inside) { dp0 = dL_dpix[pid]; dp1 = dL_dpix[HW + pid]; dp2 = dL_dpix[2 * HW + pid]; }
-    const float neg_Tf_bg = -T_final * (bg[0] * dp0 + bg[1] * dp1 + bg[2] * dp2);
+    float neg_Tf_bg, gD = 0.f;
+    if constexpr (DA) {
+        // any of the three upstream maps may be absent (NULL = zero)
+        float gA = 0.f;
+        if (inside) {
+            if (dL_dpix) { dp0 = dL_dpix[pid]; dp1 = dL_dpix[HW + pid]; dp2 = dL_dpix[2 * HW + pid]; }
+            if (dL_ddmap) gD = dL_ddmap[pid];
+            if (dL_damap) gA = dL_damap[pid];
+        }
+        neg_Tf_bg = -T_final * ((bg[0] * dp0 + bg[1] * dp1 + bg[2] * dp2) - gA);
+    } else {
+        if (inside) { dp0 = dL_dpix[pid]; dp1 = dL_dpix[HW + pid]; dp2 = dL_dpix[2 * HW + pid]; }
+        neg_Tf_bg = -T_final * (bg[0] * dp0 + bg[1] * dp1 + bg[2] * dp2);
+    }
     float ar0 = 0.f, ar1 = 0.f, ar2 = 0.f, lc0 = 0.f, lc1 = 0.f, lc2 = 0.f, last_alpha = 0.f;
+    float ar3 = 0.f, lc3 = 0.f;                                // depth channel (DA only)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t a_rec = (uint32_t)__cvta_generic_to_shared(s_rec);
-    float *const xg = s_buf_all + warp * MR_WARP_FLOATS;
+    float *const xg = s_buf_all + warp * kMrWarpFloats<DA>;
     float *const xd = xg + MR_ROWS * MR_STRIDE;
-    float *const wc = xd + MR_ROWS * MR_STRIDE;                // [3][32] dL/dpixel of the patch
-    int *const meta = reinterpret_cast<int *>(wc + 96);        // [MR_ROWS] staged slot of each parked visit
+    float *const wc = xd + MR_ROWS * MR_STRIDE;                // [3][32] dL/dpixel of the patch (DA: [4][32], + g_D)
+    int *const meta = reinterpret_cast<int *>(wc + (DA ? 128 : 96));   // [MR_ROWS] staged slot of each parked visit
     wc[lane] = dp0; wc[32 + lane] = dp1; wc[64 + lane] = dp2;
+    if constexpr (DA) wc[96 + lane] = gD;
 
     const int warp_last = __reduce_max_sync(0xffffffffu, last);
     if (lane == 0) s_max[warp] = warp_last;
@@ -599,7 +645,7 @@ blend_bwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
     auto flush = [&]() {
         __syncwarp();
         // lane (fr, fh): visit row fr, pixel rows 2 fh and 2 fh + 1 of the patch (source lanes 16 fh .. 16 fh + 15)
-        float S = 0.f, Su = 0.f, Sv = 0.f, Suu = 0.f, Suv = 0.f, Svv = 0.f, C0 = 0.f, C1 = 0.f, C2 = 0.f;
+        float S = 0.f, Su = 0.f, Sv = 0.f, Suu = 0.f, Suv = 0.f, Svv = 0.f, C0 = 0.f, C1 = 0.f, C2 = 0.f, C3 = 0.f;
 #pragma unroll
         for (int y = 0; y < 2; ++y) {
             const float4 g0 = lds128(a_rowg + 32u * y), g1 = lds128(a_rowg + 32u * y + 16);
@@ -616,17 +662,18 @@ blend_bwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
             S += r0; Su += r1; Suu += r2;
             Sv = fmaf(vy, r0, Sv); Suv = fmaf(vy, r1, Suv); Svv = fmaf(vy * vy, r0, Svv);
 #pragma unroll
-            for (int k = 0; k < 3; ++k) {
+            for (int k = 0; k < (DA ? 4 : 3); ++k) {
                 const float4 w0 = lds128(a_wrow + 128u * k + 32u * y), w1 = lds128(a_wrow + 128u * k + 32u * y + 16);
                 float acc = ds[0] * w0.x;
                 acc = fmaf(ds[1], w0.y, acc); acc = fmaf(ds[2], w0.z, acc); acc = fmaf(ds[3], w0.w, acc);
                 acc = fmaf(ds[4], w1.x, acc); acc = fmaf(ds[5], w1.y, acc); acc = fmaf(ds[6], w1.z, acc); acc = fmaf(ds[7], w1.w, acc);
-                if (k == 0) C0 += acc; else if (k == 1) C1 += acc; else C2 += acc;
+                if (k == 0) C0 += acc; else if (k == 1) C1 += acc; else if (k == 2) C2 += acc; else C3 += acc;
             }
         }
         S += __shfl_xor_sync(0xffffffffu, S, 16); Su += __shfl_xor_sync(0xffffffffu, Su, 16); Sv += __shfl_xor_sync(0xffffffffu, Sv, 16);
         Suu += __shfl_xor_sync(0xffffffffu, Suu, 16); Suv += __shfl_xor_sync(0xffffffffu, Suv, 16); Svv += __shfl_xor_sync(0xffffffffu, Svv, 16);
         C0 += __shfl_xor_sync(0xffffffffu, C0, 16); C1 += __shfl_xor_sync(0xffffffffu, C1, 16); C2 += __shfl_xor_sync(0xffffffffu, C2, 16);
+        if constexpr (DA) C3 += __shfl_xor_sync(0xffffffffu, C3, 16);
         if (fr < nbuf) {
             const uint32_t addr = a_rec + (uint32_t)meta[fr] * 48u;
             const float4 r0 = lds128(addr);                            // sx, sy, a2, b2
@@ -643,6 +690,7 @@ blend_bwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
                 if (b != 0.f) atomicAdd(dL_dmean2D + 3u * id, b);
                 if (c != 0.f) atomicAdd(dL_dmean2D + 3u * id + 1, c);
                 if (d != 0.f) atomicAdd(dL_dconic + 3u * id, d);
+                if constexpr (DA) { if (C3 != 0.f) atomicAdd(dL_ddepth + id, C3); }
             } else {
                 const float a = -0.5f * (fmaf(sxp, Sy, Suv) - syp * Su), b = -0.5f * fmaf(syp, Sy - Sv, Svv);
                 if (a != 0.f) atomicAdd(dL_dconic + 3u * id + 1, a);
@@ -670,7 +718,7 @@ blend_bwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
                 const float sx = r0.x - cx, sy = r0.y - cy;
                 const SplatCoef sc = splat_setup(sx, sy, r0.z, r0.w, r1.x, r1.y, r1.z, r1.w);
                 s_rec[3 * j] = sc.k0; s_rec[3 * j + 1] = sc.k1;
-                s_rec[3 * j + 2] = make_float4(r2.x, __uint_as_float(id), r1.y > 0.f ? 1.0f / r1.y : 0.f, 0.f);
+                s_rec[3 * j + 2] = make_float4(r2.x, __uint_as_float(id), r1.y > 0.f ? 1.0f / r1.y : 0.f, DA ? r2.y : 0.f);
                 mask8 = sc.mask8;
             }
             publish_masks<WORDS>(mask8, s_mask, h * 8 + warp);
@@ -702,12 +750,24 @@ blend_bwd2_kernel(const int2 *__restrict__ ranges, const uint32_t *__restrict__ 
                     const float rcp = rcp_approx(1.0f - alpha);         // 1 - alpha >= 0.01
                     T *= rcp;
                     dch = alpha * T;
-                    const float c0 = k1.z, c1 = k1.w, c2 = lds64(addr + 32).x;
-                    const float om = 1.f - last_alpha;
-                    ar0 = fmaf(last_alpha, lc0, om * ar0); lc0 = c0;
-                    ar1 = fmaf(last_alpha, lc1, om * ar1); lc1 = c1;
-                    ar2 = fmaf(last_alpha, lc2, om * ar2); lc2 = c2;
-                    float dL_dalpha = ((c0 - ar0) * dp0 + (c1 - ar1) * dp1 + (c2 - ar2) * dp2) * T;
+                    float dL_dalpha;
+                    if constexpr (DA) {
+                        const float4 q2 = lds128(addr + 32);           // b, id, 1/opacity, z
+                        const float c0 = k1.z, c1 = k1.w, c2 = q2.x, c3 = q2.w;
+                        const float om = 1.f - last_alpha;
+                        ar0 = fmaf(last_alpha, lc0, om * ar0); lc0 = c0;
+                        ar1 = fmaf(last_alpha, lc1, om * ar1); lc1 = c1;
+                        ar2 = fmaf(last_alpha, lc2, om * ar2); lc2 = c2;
+                        ar3 = fmaf(last_alpha, lc3, om * ar3); lc3 = c3;
+                        dL_dalpha = ((c0 - ar0) * dp0 + (c1 - ar1) * dp1 + (c2 - ar2) * dp2 + (c3 - ar3) * gD) * T;
+                    } else {
+                        const float c0 = k1.z, c1 = k1.w, c2 = lds64(addr + 32).x;
+                        const float om = 1.f - last_alpha;
+                        ar0 = fmaf(last_alpha, lc0, om * ar0); lc0 = c0;
+                        ar1 = fmaf(last_alpha, lc1, om * ar1); lc1 = c1;
+                        ar2 = fmaf(last_alpha, lc2, om * ar2); lc2 = c2;
+                        dL_dalpha = ((c0 - ar0) * dp0 + (c1 - ar1) * dp1 + (c2 - ar2) * dp2) * T;
+                    }
                     last_alpha = alpha;
                     dL_dalpha = fmaf(neg_Tf_bg, rcp, dL_dalpha);
                     gS = dL_dalpha * au;                       // D = dL/dG * G
@@ -762,7 +822,7 @@ extern "C" int splatco_blend_fwd(int64_t R, int H, int W, const float *bg, const
         blend_fwd_kernel<<<gx * gy, BLEND_THREADS, 0, (cudaStream_t)stream>>>(im.ranges, plist, rec, W, H, gx, bg, out_color, im.final_T,
                                                                              im.n_contrib, R > 0 ? im.order : nullptr);
     else
-        blend_fwd2_kernel<<<gx * gy, BLEND_THREADS, 0, (cudaStream_t)stream>>>(im.ranges, plist, rec, W, H, gx, bg, out_color, im.final_T,
+        blend_fwd2_kernel<false><<<gx * gy, BLEND_THREADS, 0, (cudaStream_t)stream>>>(im.ranges, plist, rec, W, H, gx, bg, out_color, im.final_T,
                                                                               im.n_contrib, R > 0 ? im.order : nullptr);
     SPLATCO_CHECK_LAUNCH();
     return 0;
@@ -784,8 +844,8 @@ extern "C" int splatco_blend_bwd(int P, int64_t R, int H, int W, const float *bg
     const int attr_i = current_device() & 63;
     if (!attr_dev[attr_i]) {
         SPLATCO_CHECK_CUDA(cudaFuncSetAttribute(blend_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BWD_SMEM));
-        SPLATCO_CHECK_CUDA(cudaFuncSetAttribute(blend_bwd2_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bwd2_smem<512>()));
-        SPLATCO_CHECK_CUDA(cudaFuncSetAttribute(blend_bwd2_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bwd2_smem<256>()));
+        SPLATCO_CHECK_CUDA(cudaFuncSetAttribute(blend_bwd2_kernel<512, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bwd2_smem<512>()));
+        SPLATCO_CHECK_CUDA(cudaFuncSetAttribute(blend_bwd2_kernel<256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bwd2_smem<256>()));
         attr_dev[attr_i] = 1;
     }
     const uint32_t *plist = b.vals[splatco_sorted_buffer_index(H, W)];
@@ -794,11 +854,63 @@ extern "C" int splatco_blend_bwd(int P, int64_t R, int H, int W, const float *bg
         blend_bwd_kernel<<<gx * gy, BLEND_THREADS, BWD_SMEM, (cudaStream_t)stream>>>(
             im.ranges, plist, rec, W, H, gx, bg, im.final_T, im.n_contrib, dL_dpix, dL_dmean2D, dL_dconic, dL_dopacity, dL_dcolor, im.order);
     else if (impl == 2)
-        blend_bwd2_kernel<512><<<gx * gy, BLEND_THREADS, bwd2_smem<512>(), (cudaStream_t)stream>>>(
+        blend_bwd2_kernel<512, false><<<gx * gy, BLEND_THREADS, bwd2_smem<512>(), (cudaStream_t)stream>>>(
             im.ranges, plist, rec, W, H, gx, bg, im.final_T, im.n_contrib, dL_dpix, dL_dmean2D, dL_dconic, dL_dopacity, dL_dcolor, im.order);
     else
-        blend_bwd2_kernel<256><<<gx * gy, BLEND_THREADS, bwd2_smem<256>(), (cudaStream_t)stream>>>(
+        blend_bwd2_kernel<256, false><<<gx * gy, BLEND_THREADS, bwd2_smem<256>(), (cudaStream_t)stream>>>(
             im.ranges, plist, rec, W, H, gx, bg, im.final_T, im.n_contrib, dL_dpix, dL_dmean2D, dL_dconic, dL_dopacity, dL_dcolor, im.order);
+    SPLATCO_CHECK_LAUNCH();
+    return 0;
+}
+
+// Depth / alpha maps: always the v2 kernels (splatco_blend_set_impl does not apply).
+extern "C" int splatco_blend_fwd_depth_alpha(int64_t R, int H, int W, const float *bg, const void *geom,
+                                             const void *binning, void *image, float *out_color, float *out_depth,
+                                             float *out_alpha, void *stream) {
+    SPLATCO_REQUIRE(H > 0 && W > 0 && R >= 0 && R < 0x7fffffff, "blend_fwd_depth_alpha: bad sizes");
+    SPLATCO_REQUIRE(bg && image && out_color && out_depth && out_alpha, "blend_fwd_depth_alpha: null pointer");
+    SPLATCO_REQUIRE(R == 0 || (geom && binning), "blend_fwd_depth_alpha: null workspace with R>0");
+    ImgWs im = img_view(image, H, W);
+    const int gx = ceil_div(W, TILE), gy = ceil_div(H, TILE);
+    const uint32_t *plist = nullptr;
+    const float4 *rec = nullptr;
+    if (R > 0) {
+        BinWs b = bin_view(const_cast<void *>(binning), R);
+        plist = b.vals[splatco_sorted_buffer_index(H, W)];
+        rec = reinterpret_cast<const float4 *>(geom);
+    }
+    blend_fwd2_kernel<true><<<gx * gy, BLEND_THREADS, 0, (cudaStream_t)stream>>>(
+        im.ranges, plist, rec, W, H, gx, bg, out_color, im.final_T, im.n_contrib, R > 0 ? im.order : nullptr, out_depth, out_alpha);
+    SPLATCO_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int splatco_blend_bwd_depth_alpha(int P, int64_t R, int H, int W, const float *bg, const void *geom,
+                                             const void *binning, const void *image, const float *dL_dpix,
+                                             const float *dL_ddepth_map, const float *dL_dalpha_map,
+                                             float *dL_dmean2D, float *dL_dconic, float *dL_dopacity,
+                                             float *dL_dcolor, float *dL_ddepth, void *stream) {
+    SPLATCO_REQUIRE(H > 0 && W > 0 && R >= 0 && R < 0x7fffffff && P >= 0, "blend_bwd_depth_alpha: bad sizes");
+    SPLATCO_REQUIRE(dL_dpix || dL_ddepth_map || dL_dalpha_map,
+                    "blend_bwd_depth_alpha: all three upstream gradients are NULL (use no backward)");
+    if (P == 0 || R == 0) return 0;
+    SPLATCO_REQUIRE(bg && geom && binning && image && dL_dmean2D && dL_dconic && dL_dopacity && dL_dcolor && dL_ddepth,
+                    "blend_bwd_depth_alpha: null pointer");
+    ImgWs im = img_view(const_cast<void *>(image), H, W);
+    BinWs b = bin_view(const_cast<void *>(binning), R);
+    const int gx = ceil_div(W, TILE), gy = ceil_div(H, TILE);
+    static unsigned char attr_dev[64];       // cudaFuncSetAttribute is per device
+    const int attr_i = current_device() & 63;
+    if (!attr_dev[attr_i]) {
+        SPLATCO_CHECK_CUDA(cudaFuncSetAttribute(blend_bwd2_kernel<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                (int)bwd2_smem<512, true>()));
+        attr_dev[attr_i] = 1;
+    }
+    const uint32_t *plist = b.vals[splatco_sorted_buffer_index(H, W)];
+    const float4 *rec = reinterpret_cast<const float4 *>(geom);
+    blend_bwd2_kernel<512, true><<<gx * gy, BLEND_THREADS, bwd2_smem<512, true>(), (cudaStream_t)stream>>>(
+        im.ranges, plist, rec, W, H, gx, bg, im.final_T, im.n_contrib, dL_dpix, dL_dmean2D, dL_dconic, dL_dopacity, dL_dcolor,
+        im.order, dL_ddepth_map, dL_dalpha_map, dL_ddepth);
     SPLATCO_CHECK_LAUNCH();
     return 0;
 }

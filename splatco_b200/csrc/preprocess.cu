@@ -254,6 +254,11 @@ preprocess_fwd_kernel(int P, const uint32_t *__restrict__ P_dev, const float *__
 }
 
 // ---- per-Gaussian backward chain (fp32; tolerance-compared, so the compiler may contract) --------
+// DEPTH: the blend's dL/dz_view (the one trailing argument, `const float *dL_ddepth`) is added to dL/dmeans3D through
+// dz_view/dmean = (V[2], V[6], V[10]).  It is a parameter pack, empty without DEPTH, so that preprocess_bwd_kernel<false>
+// keeps the parameter list -- and with it the code -- of the colour-only kernel.
+__device__ __forceinline__ const float *depth_grad_ptr(const float *p) { return p; }
+template <bool DEPTH, typename... DepthGrad>
 __global__ void __launch_bounds__(PRE_THREADS)
 preprocess_bwd_kernel(int P, const float *__restrict__ means3D, const float *__restrict__ scales,
                       int scale_stride, const float *__restrict__ rots, float mod,
@@ -261,7 +266,7 @@ preprocess_bwd_kernel(int P, const float *__restrict__ means3D, const float *__r
                       float tanfovy, float fx, float fy, const int32_t *__restrict__ radii,
                       const float *__restrict__ dL_dmean2D, const float *__restrict__ dL_dconic,
                       float *__restrict__ dL_dmeans3D, float *__restrict__ dL_dscales,
-                      float *__restrict__ dL_drots) {
+                      float *__restrict__ dL_drots, DepthGrad... dL_ddepth) {
     __shared__ float s_cam[32];
     stage_cam(s_cam, view, proj);
     const float *V = s_cam, *Pm = s_cam + 16;
@@ -352,6 +357,10 @@ preprocess_bwd_kernel(int P, const float *__restrict__ means3D, const float *__r
         gmx += (Pm[0] * mw - Pm[3] * mul1) * g2x + (Pm[1] * mw - Pm[3] * mul2) * g2y;
         gmy += (Pm[4] * mw - Pm[7] * mul1) * g2x + (Pm[5] * mw - Pm[7] * mul2) * g2y;
         gmz += (Pm[8] * mw - Pm[11] * mul1) * g2x + (Pm[9] * mw - Pm[11] * mul2) * g2y;
+        if constexpr (DEPTH) {
+            const float gd = depth_grad_ptr(dL_ddepth...)[i];
+            gmx = fmaf(V[2], gd, gmx); gmy = fmaf(V[6], gd, gmy); gmz = fmaf(V[10], gd, gmz);
+        }
         // Sigma = M M^T: dM = 2 dS M;  M_ak = R_ak s_k
         float dR[3][3], gsv[3];
 #pragma unroll
@@ -487,22 +496,49 @@ extern "C" int splatco_preprocess_fwd_counted(int P_max, const int32_t *P_dev, c
                                num_rendered_host, stream);
 }
 
+template <bool DEPTH>
+static int preprocess_bwd_impl(const char *name, int P, const float *means3D, const float *scales, int scale_stride,
+                               const float *rots, float scale_mod, const float *view, const float *proj, float tanfovx,
+                               float tanfovy, int H, int W, const int32_t *radii, const float *dL_dmean2D,
+                               const float *dL_dconic, float *dL_dmeans3D, float *dL_dscales, float *dL_drots,
+                               const float *dL_ddepth, void *stream) {
+    SPLATCO_REQUIRE(P >= 0 && H > 0 && W > 0, "%s: bad sizes", name);
+    if (P == 0) return 0;
+    SPLATCO_REQUIRE(means3D && scales && rots && view && proj && radii && dL_dmean2D && dL_dconic &&
+                    dL_dmeans3D && dL_dscales && dL_drots && (!DEPTH || dL_ddepth), "%s: null pointer", name);
+    SPLATCO_REQUIRE(((uintptr_t)rots & 15) == 0 && ((uintptr_t)dL_drots & 15) == 0,
+                    "%s: rotations / dL_drots must be 16-byte aligned", name);
+    const float fx = (float)W / (2.0f * tanfovx), fy = (float)H / (2.0f * tanfovy);
+    if constexpr (DEPTH)
+        preprocess_bwd_kernel<true, const float *><<<ceil_div(P, PRE_THREADS), PRE_THREADS, 0, (cudaStream_t)stream>>>(
+            P, means3D, scales, scale_stride, rots, scale_mod, view, proj, tanfovx, tanfovy, fx, fy, radii,
+            dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales, dL_drots, dL_ddepth);
+    else
+        preprocess_bwd_kernel<false><<<ceil_div(P, PRE_THREADS), PRE_THREADS, 0, (cudaStream_t)stream>>>(
+            P, means3D, scales, scale_stride, rots, scale_mod, view, proj, tanfovx, tanfovy, fx, fy, radii,
+            dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales, dL_drots);
+    SPLATCO_CHECK_LAUNCH();
+    return 0;
+}
+
 extern "C" int splatco_preprocess_bwd(int P, const float *means3D, const float *scales, int scale_stride,
                                       const float *rots, float scale_mod, const float *view,
                                       const float *proj, float tanfovx, float tanfovy, int H, int W,
                                       const int32_t *radii, const float *dL_dmean2D,
                                       const float *dL_dconic, float *dL_dmeans3D, float *dL_dscales,
                                       float *dL_drots, void *stream) {
-    SPLATCO_REQUIRE(P >= 0 && H > 0 && W > 0, "preprocess_bwd: bad sizes");
-    if (P == 0) return 0;
-    SPLATCO_REQUIRE(means3D && scales && rots && view && proj && radii && dL_dmean2D && dL_dconic &&
-                    dL_dmeans3D && dL_dscales && dL_drots, "preprocess_bwd: null pointer");
-    SPLATCO_REQUIRE(((uintptr_t)rots & 15) == 0 && ((uintptr_t)dL_drots & 15) == 0,
-                    "preprocess_bwd: rotations / dL_drots must be 16-byte aligned");
-    const float fx = (float)W / (2.0f * tanfovx), fy = (float)H / (2.0f * tanfovy);
-    preprocess_bwd_kernel<<<ceil_div(P, PRE_THREADS), PRE_THREADS, 0, (cudaStream_t)stream>>>(
-        P, means3D, scales, scale_stride, rots, scale_mod, view, proj, tanfovx, tanfovy, fx, fy, radii,
-        dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales, dL_drots);
-    SPLATCO_CHECK_LAUNCH();
-    return 0;
+    return preprocess_bwd_impl<false>("preprocess_bwd", P, means3D, scales, scale_stride, rots, scale_mod, view, proj,
+                                      tanfovx, tanfovy, H, W, radii, dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales,
+                                      dL_drots, nullptr, stream);
+}
+
+extern "C" int splatco_preprocess_bwd_depth(int P, const float *means3D, const float *scales, int scale_stride,
+                                            const float *rots, float scale_mod, const float *view,
+                                            const float *proj, float tanfovx, float tanfovy, int H, int W,
+                                            const int32_t *radii, const float *dL_dmean2D,
+                                            const float *dL_dconic, float *dL_dmeans3D, float *dL_dscales,
+                                            float *dL_drots, const float *dL_ddepth, void *stream) {
+    return preprocess_bwd_impl<true>("preprocess_bwd_depth", P, means3D, scales, scale_stride, rots, scale_mod, view,
+                                     proj, tanfovx, tanfovy, H, W, radii, dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales,
+                                     dL_drots, dL_ddepth, stream);
 }

@@ -88,7 +88,7 @@ class DecodeConfig:
     """Everything that is not a differentiable tensor input."""
     __slots__ = ("N", "K", "rc", "level", "E", "use_dist", "app_dim", "xyz_min", "xyz_max", "cam",
                  "bn_eps", "bn_momentum", "update_running", "buffers", "vis_idx", "noise", "noise_q", "noise_seed", "plan", "raster", "packed",
-                 "pending")
+                 "pending", "depth_alpha")
 
 
 # order of the differentiable parameter list handed to the autograd Function
@@ -214,7 +214,8 @@ class _FusedDecode(torch.autograd.Function):
                 with stage("decode_emit"):
                     check(L.splatco_decode_emit(C.byref(desc), _p(ws), VK, *[_p(b) for b in bufs], stream),
                           "splatco_decode_emit")
-                sp = _dgr.preprocess_speculative(*bufs, L.splatco_decode_count_ptr(_p(ws), V, cfg.rc, cfg.level), cfg.raster)
+                sp = _dgr.preprocess_speculative(*bufs, L.splatco_decode_count_ptr(_p(ws), V, cfg.rc, cfg.level), cfg.raster,
+                                                  depth_alpha=cfg.depth_alpha)
                 sp.event.synchronize()             # M, R (and V) have landed; binning + blend keep running behind it
                 M = int(counter[0])
                 if cp is not None:
@@ -619,10 +620,11 @@ DEFER_COUNT = _os.environ.get("SPLATCO_DEFER_COUNT", "1") != "0"
 
 
 def generate_neural_gaussians(viewpoint_camera, pc, visible_mask=None, is_training=False, _raster_settings=None,
-                              _scaling=None):
+                              _scaling=None, _depth_alpha=False):
     """Drop-in for gaussian_renderer.generate_neural_gaussians (reference :18-116).  `_raster_settings`
     is render()'s private hint: the GaussianRasterizationSettings it is about to rasterize the result
-    with, which lets the decode queue the rasterizer's preprocess before its own row count is known."""
+    with, which lets the decode queue the rasterizer's preprocess before its own row count is known;
+    `_depth_alpha` says whether that rasterization also produces the depth and alpha maps."""
     # the per-anchor inputs first (pc.get_scaling launches two kernels): collect_model ends by waiting for the
     # prefilter's visible-anchor count, and everything queued before that wait overlaps with the GPU's backlog
     scaling_in = _scaling if _scaling is not None else pc.get_scaling
@@ -631,6 +633,7 @@ def generate_neural_gaussians(viewpoint_camera, pc, visible_mask=None, is_traini
              and _register().splatco_decode_get_impl() == 2)
     cfg, att, app_vec, params = collect_model(pc, viewpoint_camera, visible_mask, defer_count=defer)
     cfg.raster = _raster_settings
+    cfg.depth_alpha = bool(_depth_alpha)
     # GaussianLearner.inference always passes Q = self.Q0 (0.03 while training, 0 in render.py):
     # U(-.5,.5)*Q is added to the plane features of the non-TA levels (scene/grids.py:159-164)
     Q = float(getattr(pc.feat_planes, "Q0", 0.0) or 0.0)

@@ -88,31 +88,34 @@ def _debug_sync(settings, what):
 
 class RasterState:
     """What forward leaves behind for backward and for the stage-wise parity tests."""
-    __slots__ = ("P", "PL", "R", "RL", "H", "W", "geom", "binning", "image", "radii", "radii_full")
+    __slots__ = ("P", "PL", "R", "RL", "H", "W", "geom", "binning", "image", "radii", "radii_full", "depth_alpha",
+                 "depth", "alpha")
     # P / R: Gaussians and instances of this view; PL / RL: the row counts the geometry / binning
     # workspaces were laid out for (>= P, R when the forward was queued before the counts were known)
+    # depth_alpha: the forward also produced the depth and alpha maps [1,H,W] (`depth`, `alpha`)
 
 
 class _Speculated:
     """preprocess_fwd launched by the decode on its own outputs before their row count M was known on
     the host (splatco_preprocess_fwd_counted), so that M and R come back in ONE sync."""
     __slots__ = ("tensors", "versions", "settings", "M", "PL", "R", "RL", "geom", "radii_full", "counter", "binning",
-                 "image", "color", "event")
+                 "image", "color", "event", "depth_alpha", "depth", "alpha")
 
 
 _spec_slot = threading.local()
 
 
-def preprocess_speculative(xyz_b, color_b, opacity_b, scaling_b, rot_b, count_ptr, settings):
+def preprocess_speculative(xyz_b, color_b, opacity_b, scaling_b, rot_b, count_ptr, settings, depth_alpha=False):
     """Called by the decode forward with its VK-row output buffers (row count still on the device at
     `count_ptr`).  Launches the counted preprocess and returns the pending record; the caller syncs,
-    then `publish_speculated` makes it available to the next rasterizer forward on these tensors."""
+    then `publish_speculated` makes it available to the next rasterizer forward on these tensors.
+    `depth_alpha`: the rasterizer call will ask for the depth and alpha maps, so the queued blend produces them."""
     L = _lib.lib()
     dev = xyz_b.device
     H, W = int(settings.image_height), int(settings.image_width)
     PL = int(xyz_b.shape[0])
     sp = _Speculated()
-    sp.settings, sp.PL = settings, PL
+    sp.settings, sp.PL, sp.depth_alpha = settings, PL, bool(depth_alpha)
     sp.radii_full = _lib.empty_rows(PL, None, torch.int32, dev)
     sp.geom = _lib.empty_u8(L.splatco_geom_bytes(PL), dev)
     sp.counter = _pinned_counter(dev, 1)
@@ -130,7 +133,7 @@ def preprocess_speculative(xyz_b, color_b, opacity_b, scaling_b, rot_b, count_pt
     # host learns M and R the GPU is already working on them instead of idling through the host-side
     # bookkeeping that follows the sync.  A wrong guess (R larger than the buffers) is detected after the
     # sync and the two stages are simply re-run (publish_speculated).
-    sp.binning = sp.image = sp.color = None
+    sp.binning = sp.image = sp.color = sp.depth = sp.alpha = None
     sp.RL = 0
     guess = _r_guess.get((H, W))
     if guess:
@@ -157,8 +160,15 @@ def _queue_binning_blend(sp, dev, H, W):
         check(L.splatco_binning(sp.PL, sp.RL, H, W, ptr(sp.radii_full), ptr(sp.geom), ptr(sp.binning), ptr(sp.image),
                                 stream), "splatco_binning")
     with stage("blend_fwd"):
-        check(L.splatco_blend_fwd(sp.RL, H, W, ptr(_f32c(settings.bg)), ptr(sp.geom), ptr(sp.binning), ptr(sp.image),
-                                  ptr(sp.color), stream), "splatco_blend_fwd")
+        if sp.depth_alpha:
+            sp.depth = torch.empty((1, H, W), dtype=torch.float32, device=dev)
+            sp.alpha = torch.empty((1, H, W), dtype=torch.float32, device=dev)
+            check(L.splatco_blend_fwd_depth_alpha(sp.RL, H, W, ptr(_f32c(settings.bg)), ptr(sp.geom), ptr(sp.binning),
+                                                  ptr(sp.image), ptr(sp.color), ptr(sp.depth), ptr(sp.alpha), stream),
+                  "splatco_blend_fwd_depth_alpha")
+        else:
+            check(L.splatco_blend_fwd(sp.RL, H, W, ptr(_f32c(settings.bg)), ptr(sp.geom), ptr(sp.binning), ptr(sp.image),
+                                      ptr(sp.color), stream), "splatco_blend_fwd")
 
 
 def publish_speculated(sp, M, outs):
@@ -177,13 +187,13 @@ def publish_speculated(sp, M, outs):
     _spec_slot.sp = sp
 
 
-def _take_speculated(means3D, colors, opacities, scales, rotations, settings):
+def _take_speculated(means3D, colors, opacities, scales, rotations, settings, depth_alpha=False):
     sp = getattr(_spec_slot, "sp", None)
     if sp is None:
         return None
     _spec_slot.sp = None
     ins = (means3D, colors, opacities, scales, rotations)
-    if sp.settings is not settings or sp.M != int(means3D.shape[0]):
+    if sp.settings is not settings or sp.M != int(means3D.shape[0]) or sp.depth_alpha != depth_alpha:
         return None
     for t, u, v in zip(ins, sp.tensors, sp.versions):
         # same memory, same shape, not written to since the decode produced it
@@ -192,8 +202,10 @@ def _take_speculated(means3D, colors, opacities, scales, rotations, settings):
     return sp
 
 
-def rasterize_forward_state(means3D, colors, opacities, scales, rotations, settings) -> tuple:
-    """Forward pass; returns (color [3,H,W], radii int32 [P], RasterState)."""
+def rasterize_forward_state(means3D, colors, opacities, scales, rotations, settings, depth_alpha=False) -> tuple:
+    """Forward pass; returns (color [3,H,W], radii int32 [P], RasterState).  With depth_alpha the state also
+    holds the depth and alpha maps [1,H,W] (`st.depth`, `st.alpha`)."""
+    depth_alpha = bool(depth_alpha)
     L = _lib.lib()
     _require_cuda(means3D, colors, opacities, scales, rotations, settings.bg, settings.viewmatrix,
                   settings.projmatrix)
@@ -203,13 +215,17 @@ def rasterize_forward_state(means3D, colors, opacities, scales, rotations, setti
     bg = _f32c(settings.bg)
     st = RasterState()
     st.P, st.PL, st.H, st.W = P, P, H, W
-    sp = _take_speculated(means3D, colors, opacities, scales, rotations, settings)
+    st.depth_alpha, st.depth, st.alpha = depth_alpha, None, None
+    sp = _take_speculated(means3D, colors, opacities, scales, rotations, settings, depth_alpha)
     if P == 0:
         st.R = st.RL = 0
         st.geom = st.binning = None
         st.image = torch.empty(L.splatco_image_bytes(H, W), dtype=torch.uint8, device=dev)
         st.radii = st.radii_full = torch.empty(0, dtype=torch.int32, device=dev)
         color = bg.reshape(3, 1, 1).expand(3, H, W).contiguous()
+        if depth_alpha:
+            st.depth = torch.zeros((1, H, W), dtype=torch.float32, device=dev)
+            st.alpha = torch.zeros((1, H, W), dtype=torch.float32, device=dev)
         return color, st.radii, st
     stream = _stream_ptr(dev)
     with _lib.on_device(dev):
@@ -218,6 +234,7 @@ def rasterize_forward_state(means3D, colors, opacities, scales, rotations, setti
             st.PL, st.R, st.RL = sp.PL, sp.R, sp.RL
             st.geom, st.binning, st.image, st.radii_full = sp.geom, sp.binning, sp.image, sp.radii_full
             st.radii = sp.radii_full[:P]
+            st.depth, st.alpha = sp.depth, sp.alpha
             _debug_sync(settings, "forward")
             return sp.color, st.radii, st
         if sp is not None:
@@ -251,67 +268,101 @@ def rasterize_forward_state(means3D, colors, opacities, scales, rotations, setti
         _debug_sync(settings, "binning")
         color = torch.empty((3, H, W), dtype=torch.float32, device=dev)
         with stage("blend_fwd"):
-            check(L.splatco_blend_fwd(R, H, W, ptr(bg), ptr(geom), ptr(binning), ptr(image), ptr(color), stream),
-                  "splatco_blend_fwd")
+            if depth_alpha:
+                st.depth = torch.empty((1, H, W), dtype=torch.float32, device=dev)
+                st.alpha = torch.empty((1, H, W), dtype=torch.float32, device=dev)
+                check(L.splatco_blend_fwd_depth_alpha(R, H, W, ptr(bg), ptr(geom), ptr(binning), ptr(image), ptr(color),
+                                                      ptr(st.depth), ptr(st.alpha), stream), "splatco_blend_fwd_depth_alpha")
+            else:
+                check(L.splatco_blend_fwd(R, H, W, ptr(bg), ptr(geom), ptr(binning), ptr(image), ptr(color), stream),
+                      "splatco_blend_fwd")
         _debug_sync(settings, "blend_fwd")
     st.R, st.RL, st.geom, st.binning, st.image, st.radii, st.radii_full = R, R, geom, binning, image, radii, radii_full
     return color, radii, st
 
 
-def rasterize_backward_state(st: RasterState, grad_color, means3D, scales, rotations, settings):
-    """Backward pass; returns dict of gradients (all fp32, same row count as the inputs)."""
+def rasterize_backward_state(st: RasterState, grad_color, means3D, scales, rotations, settings, grad_depth=None,
+                             grad_alpha=None):
+    """Backward pass; returns dict of gradients (all fp32, same row count as the inputs).
+    grad_depth / grad_alpha ([1,H,W] or None) need a depth_alpha forward.  With both None this is the colour-only
+    backward (splatco_blend_bwd + splatco_preprocess_bwd); with either given, splatco_blend_bwd_depth_alpha also
+    yields dL/dz_view per Gaussian (returned as "depth"), which splatco_preprocess_bwd_depth adds to dL/dmeans3D, and
+    grad_color may be None.  Absent upstream gradients are passed as NULL (zero)."""
+    da = grad_depth is not None or grad_alpha is not None
+    if da and not st.depth_alpha:
+        raise RuntimeError("depth / alpha gradients need a forward with depth_alpha=True")
     L = _lib.lib()
     dev = means3D.device
     P, R, H, W = st.P, st.RL, st.H, st.W          # RL: the binning workspace's layout size
-    # two allocations, two split calls: [mean2D 3 | conic 3 | opacity 1 | colour 3] is zero-filled for the blend's
-    # REDs, [means3D 3 | scales 3 | rotations 4] is overwritten by preprocess_bwd (rotations stay 16-byte aligned)
-    a, b_, c, d = torch.zeros(_lib.bucket(10 * P), dtype=torch.float32, device=dev)[:10 * P].split_with_sizes([3 * P, 3 * P, P, 3 * P])
-    g_mean2D, g_conic, g_opac, g_color = a.view(P, 3), b_.view(P, 3), c.view(P, 1), d.view(P, 3)
+    # two allocations, two split calls: [mean2D 3 | conic 3 | opacity 1 | colour 3 (| depth 1)] is zero-filled for the
+    # blend's REDs, [means3D 3 | scales 3 | rotations 4] is overwritten by preprocess_bwd (rotations stay 16-byte aligned)
+    nz = 11 if da else 10
+    parts = torch.zeros(_lib.bucket(nz * P), dtype=torch.float32, device=dev)[:nz * P].split_with_sizes(
+        [3 * P, 3 * P, P, 3 * P] + ([P] if da else []))
+    g_mean2D, g_conic, g_opac, g_color = parts[0].view(P, 3), parts[1].view(P, 3), parts[2].view(P, 1), parts[3].view(P, 3)
+    g_depth = parts[4] if da else None
     e, f, g_ = _lib.empty_rows(12 * P, None, torch.float32, dev).split_with_sizes([4 * P, 4 * P, 4 * P])
     g_rots, g_means3D, g_scales = e.view(P, 4), f[:3 * P].view(P, 3), g_[:3 * P].view(P, 3)
+    out = dict(means3D=g_means3D, means2D=g_mean2D, colors=g_color, opacities=g_opac, scales=g_scales,
+               rotations=g_rots, conic=g_conic)
+    if da:
+        out["depth"] = g_depth
     if P == 0:
-        return dict(means3D=g_means3D, means2D=g_mean2D, colors=g_color, opacities=g_opac,
-                    scales=g_scales, rotations=g_rots, conic=g_conic)
+        return out
     means3D = _f32c(means3D)
     rotations = _f32c(rotations)
     scales, sstride = _rows_f32(scales, 3)
-    grad_color = _f32c(grad_color)
     bg = _f32c(settings.bg)
     view = _f32c(settings.viewmatrix)
     proj = _f32c(settings.projmatrix)
     stream = _stream_ptr(dev)
+    ws = (ptr(bg), ptr(st.geom), ptr(st.binning), ptr(st.image))
+    blend_out = (ptr(g_mean2D), ptr(g_conic), ptr(g_opac), ptr(g_color))
+    pre_args = (P, ptr(means3D), ptr(scales), sstride, ptr(rotations), float(settings.scale_modifier), ptr(view),
+                ptr(proj), float(settings.tanfovx), float(settings.tanfovy), H, W, ptr(st.radii), ptr(g_mean2D),
+                ptr(g_conic), ptr(g_means3D), ptr(g_scales), ptr(g_rots))
     with _lib.on_device(dev):
         with stage("blend_bwd"):
-          check(L.splatco_blend_bwd(P, R, H, W, ptr(bg), ptr(st.geom), ptr(st.binning), ptr(st.image),
-                                  ptr(grad_color), ptr(g_mean2D), ptr(g_conic), ptr(g_opac), ptr(g_color),
-                                  stream), "splatco_blend_bwd")
+            if da:
+                maps = [None if t is None else _f32c(t) for t in (grad_color, grad_depth, grad_alpha)]
+                check(L.splatco_blend_bwd_depth_alpha(P, R, H, W, *ws, *[ptr(t) for t in maps], *blend_out, ptr(g_depth),
+                                                      stream), "splatco_blend_bwd_depth_alpha")
+            else:
+                grad_color = _f32c(grad_color)
+                check(L.splatco_blend_bwd(P, R, H, W, *ws, ptr(grad_color), *blend_out, stream), "splatco_blend_bwd")
         _debug_sync(settings, "blend_bwd")
         with stage("preprocess_bwd"):
-          check(L.splatco_preprocess_bwd(P, ptr(means3D), ptr(scales), sstride, ptr(rotations),
-                                       float(settings.scale_modifier), ptr(view), ptr(proj),
-                                       float(settings.tanfovx), float(settings.tanfovy), H, W, ptr(st.radii),
-                                       ptr(g_mean2D), ptr(g_conic), ptr(g_means3D), ptr(g_scales), ptr(g_rots),
-                                       stream), "splatco_preprocess_bwd")
+            if da:
+                check(L.splatco_preprocess_bwd_depth(*pre_args, ptr(g_depth), stream), "splatco_preprocess_bwd_depth")
+            else:
+                check(L.splatco_preprocess_bwd(*pre_args, stream), "splatco_preprocess_bwd")
         _debug_sync(settings, "preprocess_bwd")
-    return dict(means3D=g_means3D, means2D=g_mean2D, colors=g_color, opacities=g_opac, scales=g_scales,
-                rotations=g_rots, conic=g_conic)
+    return out
+
+
+def _check_supported(sh, cov3Ds_precomp):
+    if sh is not None and sh.numel() > 0:
+        raise NotImplementedError("splatco_b200: SH colours are not on SplatCo's path (it passes colors_precomp)")
+    if cov3Ds_precomp is not None and cov3Ds_precomp.numel() > 0:
+        raise NotImplementedError("splatco_b200: cov3D_precomp is not on SplatCo's path (it passes scales+rotations)")
+
+
+def _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations):
+    ctx.raster_settings = raster_settings
+    ctx.state = st
+    ctx.save_for_backward(means3D, scales, rotations)
+    ctx.mark_non_differentiable(radii)
+    ctx.set_materialize_grads(False)          # no zero-filled gradient tensor for `radii` (or an unused map)
 
 
 class _RasterizeGaussians(torch.autograd.Function):
     @staticmethod
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                 raster_settings):
-        if sh is not None and sh.numel() > 0:
-            raise NotImplementedError("splatco_b200: SH colours are not on SplatCo's path (it passes colors_precomp)")
-        if cov3Ds_precomp is not None and cov3Ds_precomp.numel() > 0:
-            raise NotImplementedError("splatco_b200: cov3D_precomp is not on SplatCo's path (it passes scales+rotations)")
+        _check_supported(sh, cov3Ds_precomp)
         color, radii, st = rasterize_forward_state(means3D, colors_precomp, opacities, scales, rotations,
                                                    raster_settings)
-        ctx.raster_settings = raster_settings
-        ctx.state = st
-        ctx.save_for_backward(means3D, scales, rotations)
-        ctx.mark_non_differentiable(radii)
-        ctx.set_materialize_grads(False)          # no zero-filled gradient tensor for `radii`
+        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations)
         return color, radii
 
     @staticmethod
@@ -331,6 +382,32 @@ def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales,
                                      cov3Ds_precomp, raster_settings)
 
 
+class _RasterizeGaussiansDepthAlpha(torch.autograd.Function):
+    """_RasterizeGaussians that also returns the depth and alpha maps [1,H,W] (see GaussianRasterizer.forward)."""
+
+    @staticmethod
+    def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
+                raster_settings):
+        _check_supported(sh, cov3Ds_precomp)
+        color, radii, st = rasterize_forward_state(means3D, colors_precomp, opacities, scales, rotations,
+                                                   raster_settings, depth_alpha=True)
+        depth, alpha = st.depth, st.alpha
+        st.depth = st.alpha = None                  # the state outlives the outputs in ctx; it does not need them
+        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations)
+        return color, radii, depth, alpha
+
+    @staticmethod
+    def backward(ctx, grad_out_color, _grad_radii, grad_depth, grad_alpha):
+        if grad_out_color is None and grad_depth is None and grad_alpha is None:
+            return (None,) * 9
+        means3D, scales, rotations = ctx.saved_tensors
+        # both map gradients None: exactly the colour-only backward (splatco_blend_bwd + splatco_preprocess_bwd)
+        g = rasterize_backward_state(ctx.state, grad_out_color, means3D, scales, rotations, ctx.raster_settings,
+                                     grad_depth=grad_depth, grad_alpha=grad_alpha)
+        return (g["means3D"], g["means2D"], None, g["colors"], g["opacities"], g["scales"], g["rotations"],
+                None, None)
+
+
 class GaussianRasterizer(nn.Module):
     def __init__(self, raster_settings: GaussianRasterizationSettings):
         super().__init__()
@@ -340,13 +417,20 @@ class GaussianRasterizer(nn.Module):
         raise NotImplementedError("splatco_b200: markVisible is not on SplatCo's path (use visible_filter)")
 
     def forward(self, means3D, means2D, opacities, shs=None, colors_precomp=None, scales=None, rotations=None,
-                cov3D_precomp=None):
+                cov3D_precomp=None, *, depth_alpha=False):
+        """(color [3,H,W], radii [P]); with depth_alpha=True (color, radii, depth [1,H,W], alpha [1,H,W]):
+        depth = sum_i z_i alpha_i T_i, the accumulated view-space depth with background 0, and alpha = 1 - T_final,
+        both from the walk that forms the colour and both differentiable.  The expected (normalised) depth is
+        depth / alpha where alpha > 0; the caller forms it."""
         raster_settings = self.raster_settings
         if (shs is None and colors_precomp is None) or (shs is not None and colors_precomp is not None):
             raise Exception('Please provide excatly one of either SHs or precomputed colors!')
         if ((scales is None or rotations is None) and cov3D_precomp is None) or \
                 ((scales is not None or rotations is not None) and cov3D_precomp is not None):
             raise Exception('Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!')
+        if depth_alpha:
+            return _RasterizeGaussiansDepthAlpha.apply(means3D, means2D, shs, colors_precomp, opacities, scales,
+                                                       rotations, cov3D_precomp, raster_settings)
         return rasterize_gaussians(means3D, means2D, shs, colors_precomp, opacities, scales, rotations,
                                    cov3D_precomp, raster_settings)
 

@@ -88,18 +88,22 @@ def _get_rotation(pc):
 
 
 def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, scaling_modifier=1.0, visible_mask=None,
-           retain_grad=False):
-    """Render the scene.  Background tensor (bg_color) must be on GPU!"""
+           retain_grad=False, *, depth_alpha=False):
+    """Render the scene.  Background tensor (bg_color) must be on GPU!
+
+    depth_alpha=True also returns, under "depth" and "alpha", the differentiable maps [1,H,W]
+    depth = sum_i z_i alpha_i T_i (accumulated view-space depth, background 0) and alpha = 1 - T_final, from the
+    same front-to-back walk as the image.  The expected depth is depth / alpha where alpha > 0; the caller forms it."""
     is_training = pc.get_color_mlp.training
     settings = _settings(viewpoint_camera, pipe, bg_color, scaling_modifier)
     if is_training:
         xyz, color, opacity, scaling, rot, neural_opacity, mask = generate_neural_gaussians(
             viewpoint_camera, pc, visible_mask, is_training=is_training, _raster_settings=settings,
-            _scaling=_get_scaling(pc, remember=False))
+            _scaling=_get_scaling(pc, remember=False), _depth_alpha=depth_alpha)
     else:
         xyz, color, opacity, scaling, rot = generate_neural_gaussians(
             viewpoint_camera, pc, visible_mask, is_training=is_training, _raster_settings=settings,
-            _scaling=_get_scaling(pc, remember=False))
+            _scaling=_get_scaling(pc, remember=False), _depth_alpha=depth_alpha)
 
     # zero tensor whose .grad receives the 2D (screen-space) mean gradients (reference :133-138)
     # (the reference adds `+ 0` to make it a non-leaf and calls retain_grad(); a leaf holds the same .grad after backward
@@ -107,20 +111,27 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, scaling_modifier=
     screenspace_points = torch.zeros_like(xyz, dtype=pc.get_anchor.dtype, requires_grad=True, device="cuda")
 
     rasterizer = GaussianRasterizer(raster_settings=settings)
-    rendered_image, radii = rasterizer(
-        means3D=xyz,
-        means2D=screenspace_points,
-        shs=None,
-        colors_precomp=color,
-        opacities=opacity,
-        scales=scaling,
-        rotations=rot,
-        cov3D_precomp=None)
+    if depth_alpha:
+        rendered_image, radii, depth, alpha = rasterizer(
+            means3D=xyz, means2D=screenspace_points, shs=None, colors_precomp=color, opacities=opacity, scales=scaling,
+            rotations=rot, cov3D_precomp=None, depth_alpha=True)
+    else:
+        rendered_image, radii = rasterizer(
+            means3D=xyz,
+            means2D=screenspace_points,
+            shs=None,
+            colors_precomp=color,
+            opacities=opacity,
+            scales=scaling,
+            rotations=rot,
+            cov3D_precomp=None)
 
     out = {"render": rendered_image,
            "viewspace_points": screenspace_points,
            "visibility_filter": radii > 0,
            "radii": radii}
+    if depth_alpha:
+        out.update({"depth": depth, "alpha": alpha})
     if is_training:
         out.update({"selection_mask": mask, "neural_opacity": neural_opacity, "scaling": scaling})
     return out
