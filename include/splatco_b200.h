@@ -188,6 +188,23 @@ int splatco_preprocess_bwd_depth(int P, const float *means3D, const float *scale
                                  const float *dL_dmean2D, const float *dL_dconic, float *dL_dmeans3D,
                                  float *dL_dscales, float *dL_drots, const float *dL_ddepth, void *stream);
 
+/* ---- camera gradients ---------------------------------------------------------------------------
+ * Both camera entry points WRITE (do not accumulate) their camera gradient, reduced in a fixed order: the same inputs
+ * give bitwise the same result.  ws: caller-owned scratch of splatco_camera_grad_ws_bytes(n) bytes, n = P Gaussians
+ * for the preprocess backward, n = V visible anchors for the decode backward.  Neither needs it zeroed. */
+size_t splatco_camera_grad_ws_bytes(int n);
+/* preprocess_bwd_camera: the per-Gaussian outputs of splatco_preprocess_bwd (dL_ddepth NULL) or of
+ * splatco_preprocess_bwd_depth (dL_ddepth given), computed by the same kernels, plus dL_dview[16] and dL_dproj[16]:
+ * the gradients with respect to the 16 floats of view and proj as the kernels read them.  The forward never reads
+ * view[3,7,11,15] or proj[2,6,10,14]; their gradients are 0.  Clamped t.x / t.y (beyond 1.3 tanfov) count as
+ * constants, as in the per-Gaussian backward. */
+int splatco_preprocess_bwd_camera(int P, const float *means3D, const float *scales, int scale_stride,
+                                  const float *rots, float scale_mod, const float *view, const float *proj,
+                                  float tanfovx, float tanfovy, int H, int W, const int32_t *radii,
+                                  const float *dL_dmean2D, const float *dL_dconic, float *dL_dmeans3D,
+                                  float *dL_dscales, float *dL_drots, const float *dL_ddepth, void *ws,
+                                  float *dL_dview, float *dL_dproj, void *stream);
+
 /* ---- anchor decode: replaces generate_neural_gaussians -----------------------------------------
  * (gaussian_renderer/__init__.py:18-116; FeaturePlanes.forward scene/gaussian_model.py:149-169;
  * PlaneGrid scene/grids.py:146-201; heads scene/gaussian_model.py:316-337).
@@ -292,6 +309,13 @@ int splatco_decode_bwd(const splatco_decode_desc *d, const void *fwd_ws, void *b
                        const float *d_xyz, const float *d_color, const float *d_opacity,
                        const float *d_scaling, const float *d_rot, const float *d_neural_opacity,
                        const splatco_decode_grads *g, void *stream);
+/* splatco_decode_bwd (which accumulates into g) plus d_cam[3] = dL / d camera_center (written): minus the sum, over
+ * the visible anchors, of the gradient of the view direction and distance (anchor - camera_center).  ws:
+ * splatco_camera_grad_ws_bytes(V). */
+int splatco_decode_bwd_camera(const splatco_decode_desc *d, const void *fwd_ws, void *bwd_ws, int M,
+                              const float *d_xyz, const float *d_color, const float *d_opacity,
+                              const float *d_scaling, const float *d_rot, const float *d_neural_opacity,
+                              const splatco_decode_grads *g, void *ws, float *d_cam, void *stream);
 
 /* ---- TriPlaneAttention over the TA-level planes (SURVEY.md §8 row f2) ---------------------------
  * Replaces TriPlaneAttention.forward (scene/grids.py:22-64) as applied at scene/grids.py:166-169 to

@@ -49,6 +49,8 @@ SIGNATURES = {
     "splatco_blend_fwd_depth_alpha": (_i, [_i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "splatco_blend_bwd_depth_alpha": (_i, [_i, _i64, _i, _i] + [_vp] * 13),
     "splatco_preprocess_bwd_depth": (_i, [_i, _vp, _vp, _i, _vp, _f, _vp, _vp, _f, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "splatco_camera_grad_ws_bytes": (_sz, [_i]),
+    "splatco_preprocess_bwd_camera": (_i, [_i, _vp, _vp, _i, _vp, _f, _vp, _vp, _f, _f, _i, _i] + [_vp] * 11),
     # decode: descriptor / gradient structs are passed with ctypes.byref (see decode.py)
     "splatco_pack_planes": (_i, [_i, _i] + [_vp] * 7),
     "splatco_unpack_planes_add": (_i, [_i, _i] + [_vp] * 7),
@@ -65,6 +67,7 @@ SIGNATURES = {
     "splatco_decode_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "splatco_decode_emit": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "splatco_decode_bwd": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "splatco_decode_bwd_camera": (_i, [_vp, _vp, _vp, _i] + [_vp] * 10),
     "splatco_ta_fwd_ws_bytes": (_sz, [_i, _i]),
     "splatco_ta_bwd_ws_bytes": (_sz, [_i, _i]),
     "splatco_ta_fwd": (_i, [_i, _i, _i, _i] + [_vp] * 11),

@@ -1463,6 +1463,7 @@ int v2_decode_emit(const splatco_decode_desc *d, const void *ws, int M, float *x
 }  // namespace
 
 #include "decode2_bwd.cuh"
+#include "camgrad.cuh"
 
 namespace splatco {
 __global__ void __launch_bounds__(256)
@@ -1476,6 +1477,27 @@ dec2_untile_kernel(int V, int nch, int DP, int LDX, const float4 *__restrict__ X
         val = reinterpret_cast<const float *>(XT + ((size_t)(v >> 7) * nch) * D2_ROWS + (v & 127))[d2_tile_idx(uc)];
     }
     out[t] = val;
+}
+
+// dL/dcamera_center = -sum over the visible anchors of the direction / distance gradient the input kernels add to
+// dL/danchor (dec_bwd_inputs_kernel, dec2_bwd_inputs_kernel; same formula, same operands): one thread per anchor reads
+// (dir, dist) and its upstream gradient as two 16-byte cells and leaves one partial per CTA (camgrad.cuh).
+//   nch > 0: v2 tile layout (XT / DUT, chunk D2_DIR_CH of a tile of nch chunks);  nch == 0: v1 rows (XIN / DX, columns FD..FD+3)
+__global__ void __launch_bounds__(CAM_ROWS)
+dec_camera_grad_kernel(int V, int nch, const float4 *__restrict__ X, const float4 *__restrict__ G, float *__restrict__ part) {
+    const int v = blockIdx.x * CAM_ROWS + threadIdx.x;
+    float cg[CAM_COLS];
+#pragma unroll
+    for (int c = 0; c < CAM_COLS; ++c) cg[c] = 0.f;
+    if (v < V) {
+        const size_t cell = nch > 0 ? ((size_t)(v >> 7) * nch + D2_DIR_CH) * D2_ROWS + (v & 127) : ((size_t)v * XI + FD) / 4;
+        const float4 dd = __ldg(X + cell), gd = __ldg(G + cell);
+        const float dot = dd.x * gd.x + dd.y * gd.y + dd.z * gd.z;
+        cg[0] = (gd.x - dd.x * dot) / dd.w + gd.w * dd.x;
+        cg[1] = (gd.y - dd.y * dot) / dd.w + gd.w * dd.y;
+        cg[2] = (gd.z - dd.z * dot) / dd.w + gd.w * dd.z;
+    }
+    camera_block_partial(cg, part);
 }
 }  // namespace splatco
 
@@ -1553,4 +1575,39 @@ extern "C" int splatco_decode_bwd(const splatco_decode_desc *d, const void *fwd_
     if (check_desc(d)) return -1;
     return use_v2(d->rc) ? v2_decode_bwd(d, fwd_ws, bwd_ws, M, d_xyz, d_color, d_opacity, d_scaling, d_rot, d_neural_opacity, g, stream)
                          : v1_decode_bwd(d, fwd_ws, bwd_ws, M, d_xyz, d_color, d_opacity, d_scaling, d_rot, d_neural_opacity, g, stream);
+}
+
+extern "C" int splatco_decode_bwd_camera(const splatco_decode_desc *d, const void *fwd_ws, void *bwd_ws, int M,
+                                         const float *d_xyz, const float *d_color, const float *d_opacity,
+                                         const float *d_scaling, const float *d_rot, const float *d_neural_opacity,
+                                         const splatco_decode_grads *g, void *ws, float *d_cam, void *stream) {
+    if (check_desc(d)) return -1;
+    SPLATCO_REQUIRE(d_cam && (d->V == 0 || ws), "decode_bwd_camera: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d->V == 0) {
+        SPLATCO_CHECK_CUDA(cudaMemsetAsync(d_cam, 0, 3 * sizeof(float), st));
+        return 0;
+    }
+    const bool v2 = use_v2(d->rc);
+    const int rc = v2 ? v2_decode_bwd(d, fwd_ws, bwd_ws, M, d_xyz, d_color, d_opacity, d_scaling, d_rot, d_neural_opacity, g, stream)
+                      : v1_decode_bwd(d, fwd_ws, bwd_ws, M, d_xyz, d_color, d_opacity, d_scaling, d_rot, d_neural_opacity, g, stream);
+    if (rc) return rc;
+    const float4 *X, *G;
+    int nch = 0;
+    if (v2) {
+        const D2Dims dd = d2_dims(d2_layout_rows(d), d->rc, d->level);
+        X = f2_view(const_cast<void *>(fwd_ws), dd).XT;
+        G = b2_view(bwd_ws, dd).DUT;
+        nch = dd.nch;
+    } else {
+        const DecDims dd = dec_dims(d->V, d->rc, d->level);
+        X = reinterpret_cast<const float4 *>(fwd_view(const_cast<void *>(fwd_ws), dd).XIN);
+        G = reinterpret_cast<const float4 *>(bwd_view(bwd_ws, dd).DX);
+    }
+    const int nb = ceil_div(d->V, CAM_ROWS);
+    dec_camera_grad_kernel<<<nb, CAM_ROWS, 0, st>>>(d->V, nch, X, G, (float *)ws);
+    SPLATCO_CHECK_LAUNCH();
+    camera_sum_kernel<<<1, 1024, 0, st>>>(nb, 3, 3, -1.0f, (const float *)ws, d_cam, nullptr);
+    SPLATCO_CHECK_LAUNCH();
+    return 0;
 }

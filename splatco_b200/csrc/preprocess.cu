@@ -11,6 +11,7 @@
 // Rounding contract: the chain that decides integers (radius, rect, tiles_touched, depth key) uses
 // individually rounded __f*_rn operations in exactly the order of oracle/raster_oracle.c, so the
 // integer outputs are bit-identical to the CPU oracle regardless of nvcc's FMA contraction.
+#include "camgrad.cuh"
 #include "common.cuh"
 
 namespace splatco {
@@ -385,6 +386,113 @@ preprocess_bwd_kernel(int P, const float *__restrict__ means3D, const float *__r
     *reinterpret_cast<float4 *>(dL_drots + 4 * (size_t)i) = gq;
 }
 
+// ---- camera gradients: dL/dviewmatrix and dL/dprojmatrix -----------------------------------------------------------
+// Launched after preprocess_bwd_kernel, which stays as it is: this kernel re-derives the same chain from the same
+// inputs (formulas and evaluation order of preprocess_bwd_kernel) and reduces, per CTA, the 32 camera floats
+//     dV[4k+r]  += g[r] p~_k                         g = dL/dp_view = (dtx, dty, dtz + dL_ddepth),  p~ = (x, y, z, 1)
+//     dV[4k]    += dA[0][k] J00,   dV[4k+1] += dA[1][k] J11,   dV[4k+2] += dA[0][k] J02 + dA[1][k] J12   (k < 3)
+//     dPm[4k]   += g2x mw p~_k,    dPm[4k+1] += g2y mw p~_k,   dPm[4k+3] += -(g2x hx + g2y hy) mw^2 p~_k
+// into part[blockIdx.x][0..31] (camgrad.cuh).  The forward never reads V[3,7,11,15] or Pm[2,6,10,14]: those stay 0.
+__global__ void __launch_bounds__(PRE_THREADS)
+preprocess_bwd_camera_kernel(int P, const float *__restrict__ means3D, const float *__restrict__ scales,
+                             int scale_stride, const float *__restrict__ rots, float mod,
+                             const float *__restrict__ view, const float *__restrict__ proj, float tanfovx,
+                             float tanfovy, float fx, float fy, const int32_t *__restrict__ radii,
+                             const float *__restrict__ dL_dmean2D, const float *__restrict__ dL_dconic,
+                             const float *__restrict__ dL_ddepth, float *__restrict__ part) {
+    static_assert(PRE_THREADS == CAM_ROWS, "one camera partial per preprocess CTA");
+    __shared__ float s_cam[32];
+    stage_cam(s_cam, view, proj);
+    const float *V = s_cam, *Pm = s_cam + 16;
+    const int i = blockIdx.x * PRE_THREADS + threadIdx.x;
+    float cg[CAM_COLS];
+#pragma unroll
+    for (int c = 0; c < CAM_COLS; ++c) cg[c] = 0.f;
+    if (i < P && radii[i] > 0) {
+        const float x = means3D[3 * (size_t)i], y = means3D[3 * (size_t)i + 1], z = means3D[3 * (size_t)i + 2];
+        const float *sp = scales + (size_t)scale_stride * i;
+        const float4 q = *reinterpret_cast<const float4 *>(rots + 4 * (size_t)i);
+        const float vx = V[0] * x + V[4] * y + V[8] * z + V[12];
+        const float vy = V[1] * x + V[5] * y + V[9] * z + V[13];
+        const float vz = V[2] * x + V[6] * y + V[10] * z + V[14];
+        const float s[3] = { mod * sp[0], mod * sp[1], mod * sp[2] };
+        const float qr = q.x, qx = q.y, qy = q.z, qz = q.w;
+        float R[3][3];
+        R[0][0] = 1.f - 2.f * (qy * qy + qz * qz); R[0][1] = 2.f * (qx * qy - qr * qz); R[0][2] = 2.f * (qx * qz + qr * qy);
+        R[1][0] = 2.f * (qx * qy + qr * qz); R[1][1] = 1.f - 2.f * (qx * qx + qz * qz); R[1][2] = 2.f * (qy * qz - qr * qx);
+        R[2][0] = 2.f * (qx * qz - qr * qy); R[2][1] = 2.f * (qy * qz + qr * qx); R[2][2] = 1.f - 2.f * (qx * qx + qy * qy);
+        float M[3][3], S[3][3];
+#pragma unroll
+        for (int a = 0; a < 3; ++a)
+#pragma unroll
+            for (int k = 0; k < 3; ++k) M[a][k] = R[a][k] * s[k];
+#pragma unroll
+        for (int a = 0; a < 3; ++a)
+#pragma unroll
+            for (int b = 0; b < 3; ++b) S[a][b] = M[a][0] * M[b][0] + M[a][1] * M[b][1] + M[a][2] * M[b][2];
+        const float limx = 1.3f * tanfovx, limy = 1.3f * tanfovy;
+        const float txtz = vx / vz, tytz = vy / vz;
+        const bool clx = (txtz < -limx) || (txtz > limx), cly = (tytz < -limy) || (tytz > limy);
+        const float tx = fminf(limx, fmaxf(-limx, txtz)) * vz, ty = fminf(limy, fmaxf(-limy, tytz)) * vz;
+        const float iz = 1.f / vz, iz2 = iz * iz, iz3 = iz2 * iz;
+        const float J00 = fx * iz, J02 = -(fx * tx) * iz2, J11 = fy * iz, J12 = -(fy * ty) * iz2;
+        float A[2][3], B[2][3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            A[0][k] = J00 * V[4 * k] + J02 * V[4 * k + 2];
+            A[1][k] = J11 * V[4 * k + 1] + J12 * V[4 * k + 2];
+        }
+#pragma unroll
+        for (int r = 0; r < 2; ++r)
+#pragma unroll
+            for (int l = 0; l < 3; ++l) B[r][l] = A[r][0] * S[0][l] + A[r][1] * S[1][l] + A[r][2] * S[2][l];
+        const float a = B[0][0] * A[0][0] + B[0][1] * A[0][1] + B[0][2] * A[0][2] + 0.3f;
+        const float b = B[0][0] * A[1][0] + B[0][1] * A[1][1] + B[0][2] * A[1][2];
+        const float c = B[1][0] * A[1][0] + B[1][1] * A[1][1] + B[1][2] * A[1][2] + 0.3f;
+        const float denom = a * c - b * b;
+        const float d2inv = 1.0f / (denom * denom + 0.0000001f);
+        const float gc0 = dL_dconic[3 * (size_t)i], gc1 = dL_dconic[3 * (size_t)i + 1], gc2 = dL_dconic[3 * (size_t)i + 2];
+        const float dL_da = d2inv * (-c * c * gc0 + 2.f * b * c * gc1 + (denom - a * c) * gc2);
+        const float dL_dc = d2inv * (-a * a * gc2 + 2.f * a * b * gc1 + (denom - a * c) * gc0);
+        const float dL_db = d2inv * 2.f * (b * c * gc0 - (denom + 2.f * b * b) * gc1 + a * b * gc2);
+        const float G2[2][2] = { { dL_da, 0.5f * dL_db }, { 0.5f * dL_db, dL_dc } };
+        float dA[2][3];
+#pragma unroll
+        for (int r = 0; r < 2; ++r)
+#pragma unroll
+            for (int l = 0; l < 3; ++l) dA[r][l] = 2.f * (G2[r][0] * B[0][l] + G2[r][1] * B[1][l]);
+        float dJ00 = 0.f, dJ02 = 0.f, dJ11 = 0.f, dJ12 = 0.f;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            dJ00 += dA[0][k] * V[4 * k]; dJ02 += dA[0][k] * V[4 * k + 2];
+            dJ11 += dA[1][k] * V[4 * k + 1]; dJ12 += dA[1][k] * V[4 * k + 2];
+        }
+        const float dtx = clx ? 0.f : -fx * iz2 * dJ02;
+        const float dty = cly ? 0.f : -fy * iz2 * dJ12;
+        float dtz = -fx * iz2 * dJ00 - fy * iz2 * dJ11 + 2.f * fx * tx * iz3 * dJ02 + 2.f * fy * ty * iz3 * dJ12;
+        if (dL_ddepth) dtz += dL_ddepth[i];
+        const float hx = Pm[0] * x + Pm[4] * y + Pm[8] * z + Pm[12];
+        const float hy = Pm[1] * x + Pm[5] * y + Pm[9] * z + Pm[13];
+        const float hw = Pm[3] * x + Pm[7] * y + Pm[11] * z + Pm[15];
+        const float mw = 1.0f / (hw + 0.0000001f);
+        const float g2x = dL_dmean2D[3 * (size_t)i], g2y = dL_dmean2D[3 * (size_t)i + 1];
+        const float ex = g2x * mw, ey = g2y * mw, ew = -(g2x * hx + g2y * hy) * mw * mw;
+        const float ph[4] = { x, y, z, 1.f };
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            cg[4 * k] = dtx * ph[k]; cg[4 * k + 1] = dty * ph[k]; cg[4 * k + 2] = dtz * ph[k];
+            cg[16 + 4 * k] = ex * ph[k]; cg[16 + 4 * k + 1] = ey * ph[k]; cg[16 + 4 * k + 3] = ew * ph[k];
+        }
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            cg[4 * k] += dA[0][k] * J00;
+            cg[4 * k + 1] += dA[1][k] * J11;
+            cg[4 * k + 2] += dA[0][k] * J02 + dA[1][k] * J12;
+        }
+    }
+    camera_block_partial(cg, part);
+}
+
 }  // namespace splatco
 
 using namespace splatco;
@@ -541,4 +649,41 @@ extern "C" int splatco_preprocess_bwd_depth(int P, const float *means3D, const f
     return preprocess_bwd_impl<true>("preprocess_bwd_depth", P, means3D, scales, scale_stride, rots, scale_mod, view,
                                      proj, tanfovx, tanfovy, H, W, radii, dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales,
                                      dL_drots, dL_ddepth, stream);
+}
+
+extern "C" size_t splatco_camera_grad_ws_bytes(int n) { return camera_grad_ws_bytes(n); }
+
+extern "C" int splatco_preprocess_bwd_camera(int P, const float *means3D, const float *scales, int scale_stride,
+                                             const float *rots, float scale_mod, const float *view,
+                                             const float *proj, float tanfovx, float tanfovy, int H, int W,
+                                             const int32_t *radii, const float *dL_dmean2D,
+                                             const float *dL_dconic, float *dL_dmeans3D, float *dL_dscales,
+                                             float *dL_drots, const float *dL_ddepth, void *ws, float *dL_dview,
+                                             float *dL_dproj, void *stream) {
+    SPLATCO_REQUIRE(P >= 0 && H > 0 && W > 0, "preprocess_bwd_camera: bad sizes");
+    SPLATCO_REQUIRE(dL_dview && dL_dproj && (P == 0 || ws), "preprocess_bwd_camera: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (P == 0) {
+        SPLATCO_CHECK_CUDA(cudaMemsetAsync(dL_dview, 0, 16 * sizeof(float), st));
+        SPLATCO_CHECK_CUDA(cudaMemsetAsync(dL_dproj, 0, 16 * sizeof(float), st));
+        return 0;
+    }
+    // the per-Gaussian outputs: exactly the camera-off call
+    const int rc = dL_ddepth ? preprocess_bwd_impl<true>("preprocess_bwd_camera", P, means3D, scales, scale_stride, rots,
+                                                         scale_mod, view, proj, tanfovx, tanfovy, H, W, radii, dL_dmean2D,
+                                                         dL_dconic, dL_dmeans3D, dL_dscales, dL_drots, dL_ddepth, stream)
+                             : preprocess_bwd_impl<false>("preprocess_bwd_camera", P, means3D, scales, scale_stride, rots,
+                                                          scale_mod, view, proj, tanfovx, tanfovy, H, W, radii, dL_dmean2D,
+                                                          dL_dconic, dL_dmeans3D, dL_dscales, dL_drots, nullptr, stream);
+    if (rc) return rc;
+    const float fx = (float)W / (2.0f * tanfovx), fy = (float)H / (2.0f * tanfovy);
+    const int nb = ceil_div(P, PRE_THREADS);
+    float *part = (float *)ws;
+    preprocess_bwd_camera_kernel<<<nb, PRE_THREADS, 0, st>>>(P, means3D, scales, scale_stride, rots, scale_mod, view, proj,
+                                                             tanfovx, tanfovy, fx, fy, radii, dL_dmean2D, dL_dconic,
+                                                             dL_ddepth, part);
+    SPLATCO_CHECK_LAUNCH();
+    camera_sum_kernel<<<1, 1024, 0, st>>>(nb, 32, 16, 1.0f, part, dL_dview, dL_dproj);
+    SPLATCO_CHECK_LAUNCH();
+    return 0;
 }

@@ -88,7 +88,7 @@ class DecodeConfig:
     """Everything that is not a differentiable tensor input."""
     __slots__ = ("N", "K", "rc", "level", "E", "use_dist", "app_dim", "xyz_min", "xyz_max", "cam",
                  "bn_eps", "bn_momentum", "update_running", "buffers", "vis_idx", "noise", "noise_q", "noise_seed", "plan", "raster", "packed",
-                 "pending", "depth_alpha")
+                 "pending", "depth_alpha", "cam_grad")
 
 
 # order of the differentiable parameter list handed to the autograd Function
@@ -168,6 +168,10 @@ class _FusedDecode(torch.autograd.Function):
     @staticmethod
     def forward(ctx, cfg: DecodeConfig, anchor_feat, anchor, offset, scaling, att_xy, att_xz, att_yz, app_vec,
                 *params):
+        # cfg.cam_grad: the last input is the camera centre (the tensor cfg.cam was read from), which wants a gradient
+        if cfg.cam_grad:
+            ctx.cam_meta = (params[-1].shape, params[-1].dtype)
+            params = params[:-1]
         L = _register()
         dev = anchor.device
         # kernels read fp32 contiguous memory; tensors that already are (the normal case) are used in place
@@ -272,12 +276,14 @@ class _FusedDecode(torch.autograd.Function):
             got = _gradacc.acquire(dev, reqs)
         slots = _grad_slots(nl)
         vals = [None] * _NGRAD
-        rets = [None] * len(origs)
+        rets = [None] * len(origs)                 # (a camera centre input is last; its gradient is appended below)
         for n, (ptr_n, ret) in zip(where, got):
             vals[slots[n]] = ptr_n
             rets[n] = ret if need[n] else None
         del got
         gd = _GradPtrs(*vals)                  # same memory layout as splatco_decode_grads (all pointers)
+        cam = cfg.cam_grad and ctx.needs_input_grad[-1]
+        d_cam = torch.zeros(3, dtype=torch.float32, device=dev) if cam else None
         if V > 0:
             ups = [_c(t) if t is not None else None for t in (g_xyz, g_color, g_opacity, g_scl, g_rot, g_nopac)]
             if M > 0:
@@ -287,9 +293,17 @@ class _FusedDecode(torch.autograd.Function):
             with _lib.on_device(dev):
                 bws = _lib.empty_u8(L.splatco_decode_bwd_ws_bytes(ctx.V_rows, cfg.rc, cfg.level), dev)
                 with stage("decode_bwd"):
-                    check(L.splatco_decode_bwd(C.byref(desc), _p(ctx.ws), _p(bws), M, *[_p(u) for u in ups],
-                                               gd, stream), "splatco_decode_bwd")
-        return (None, *rets)
+                    if cam:
+                        cam_ws = _lib.empty_u8(L.splatco_camera_grad_ws_bytes(V), dev)
+                        check(L.splatco_decode_bwd_camera(C.byref(desc), _p(ctx.ws), _p(bws), M, *[_p(u) for u in ups],
+                                                          gd, _p(cam_ws), _p(d_cam), stream), "splatco_decode_bwd_camera")
+                    else:
+                        check(L.splatco_decode_bwd(C.byref(desc), _p(ctx.ws), _p(bws), M, *[_p(u) for u in ups],
+                                                   gd, stream), "splatco_decode_bwd")
+        if not cfg.cam_grad:
+            return (None, *rets)
+        shape, dtype = ctx.cam_meta
+        return (None, *rets, d_cam.to(dtype).reshape(shape) if cam else None)
 
 
 def _bn_lin(seq):
@@ -634,6 +648,10 @@ def generate_neural_gaussians(viewpoint_camera, pc, visible_mask=None, is_traini
     cfg, att, app_vec, params = collect_model(pc, viewpoint_camera, visible_mask, defer_count=defer)
     cfg.raster = _raster_settings
     cfg.depth_alpha = bool(_depth_alpha)
+    # a camera centre that requires grad (a pose being optimised) becomes a differentiable input of the decode
+    cam = viewpoint_camera.camera_center
+    cam_in = (cam,) if torch.is_grad_enabled() and cam.requires_grad else ()
+    cfg.cam_grad = bool(cam_in)
     # GaussianLearner.inference always passes Q = self.Q0 (0.03 while training, 0 in render.py):
     # U(-.5,.5)*Q is added to the plane features of the non-TA levels (scene/grids.py:159-164)
     Q = float(getattr(pc.feat_planes, "Q0", 0.0) or 0.0)
@@ -646,7 +664,7 @@ def generate_neural_gaussians(viewpoint_camera, pc, visible_mask=None, is_traini
         cfg.noise_q = Q
         cfg.noise_seed = (torch.initial_seed() * 0x9E3779B97F4A7C15 + _noise_calls * 0xD1B54A32D192ED03) & 0xFFFFFFFFFFFFFFFF
     outs = _FusedDecode.apply(cfg, pc._anchor_feat, pc.get_anchor, pc._offset, scaling_in, att[0], att[1], att[2],
-                              app_vec, *params)
+                              app_vec, *params, *cam_in)
     xyz, color, opacity, scaling, rot, neural_opacity, mask = outs
     if is_training:
         return xyz, color, opacity, scaling, rot, neural_opacity, mask

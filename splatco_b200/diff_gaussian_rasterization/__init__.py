@@ -282,12 +282,14 @@ def rasterize_forward_state(means3D, colors, opacities, scales, rotations, setti
 
 
 def rasterize_backward_state(st: RasterState, grad_color, means3D, scales, rotations, settings, grad_depth=None,
-                             grad_alpha=None):
+                             grad_alpha=None, camera=False):
     """Backward pass; returns dict of gradients (all fp32, same row count as the inputs).
     grad_depth / grad_alpha ([1,H,W] or None) need a depth_alpha forward.  With both None this is the colour-only
     backward (splatco_blend_bwd + splatco_preprocess_bwd); with either given, splatco_blend_bwd_depth_alpha also
     yields dL/dz_view per Gaussian (returned as "depth"), which splatco_preprocess_bwd_depth adds to dL/dmeans3D, and
-    grad_color may be None.  Absent upstream gradients are passed as NULL (zero)."""
+    grad_color may be None.  Absent upstream gradients are passed as NULL (zero).
+    camera=True: splatco_preprocess_bwd_camera replaces the preprocess backward (same per-Gaussian outputs) and the dict
+    also holds "viewmatrix" and "projmatrix", fp32 [4,4]: the gradients of the contiguous fp32 copies the kernels read."""
     da = grad_depth is not None or grad_alpha is not None
     if da and not st.depth_alpha:
         raise RuntimeError("depth / alpha gradients need a forward with depth_alpha=True")
@@ -307,6 +309,9 @@ def rasterize_backward_state(st: RasterState, grad_color, means3D, scales, rotat
                rotations=g_rots, conic=g_conic)
     if da:
         out["depth"] = g_depth
+    if camera:
+        g_cam = torch.zeros(32, dtype=torch.float32, device=dev) if P == 0 else torch.empty(32, dtype=torch.float32, device=dev)
+        out["viewmatrix"], out["projmatrix"] = g_cam[:16].view(4, 4), g_cam[16:].view(4, 4)
     if P == 0:
         return out
     means3D = _f32c(means3D)
@@ -332,7 +337,11 @@ def rasterize_backward_state(st: RasterState, grad_color, means3D, scales, rotat
                 check(L.splatco_blend_bwd(P, R, H, W, *ws, ptr(grad_color), *blend_out, stream), "splatco_blend_bwd")
         _debug_sync(settings, "blend_bwd")
         with stage("preprocess_bwd"):
-            if da:
+            if camera:
+                cam_ws = _lib.empty_u8(L.splatco_camera_grad_ws_bytes(P), dev)
+                check(L.splatco_preprocess_bwd_camera(*pre_args, ptr(g_depth), ptr(cam_ws), ptr(out["viewmatrix"]),
+                                                      ptr(out["projmatrix"]), stream), "splatco_preprocess_bwd_camera")
+            elif da:
                 check(L.splatco_preprocess_bwd_depth(*pre_args, ptr(g_depth), stream), "splatco_preprocess_bwd_depth")
             else:
                 check(L.splatco_preprocess_bwd(*pre_args, stream), "splatco_preprocess_bwd")
@@ -408,6 +417,39 @@ class _RasterizeGaussiansDepthAlpha(torch.autograd.Function):
                 None, None)
 
 
+class _RasterizeGaussiansCamera(torch.autograd.Function):
+    """_RasterizeGaussians (depth_alpha False) or _RasterizeGaussiansDepthAlpha (True) with the view and projection
+    matrices of the settings as differentiable inputs: GaussianRasterizer.forward routes here when either of them
+    requires grad.  Their gradients are taken with respect to the [4,4] elements, whatever dtype and strides the
+    tensors have; `campos` gets none (there are no SH colours)."""
+
+    @staticmethod
+    def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
+                raster_settings, viewmatrix, projmatrix, depth_alpha):
+        _check_supported(sh, cov3Ds_precomp)
+        color, radii, st = rasterize_forward_state(means3D, colors_precomp, opacities, scales, rotations,
+                                                   raster_settings, depth_alpha=depth_alpha)
+        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations)
+        ctx.cam_dtypes = (viewmatrix.dtype, projmatrix.dtype)
+        if not depth_alpha:
+            return color, radii
+        depth, alpha = st.depth, st.alpha
+        st.depth = st.alpha = None
+        return color, radii, depth, alpha
+
+    @staticmethod
+    def backward(ctx, grad_out_color, _grad_radii, grad_depth=None, grad_alpha=None):
+        if grad_out_color is None and grad_depth is None and grad_alpha is None:
+            return (None,) * 12
+        means3D, scales, rotations = ctx.saved_tensors
+        g = rasterize_backward_state(ctx.state, grad_out_color, means3D, scales, rotations, ctx.raster_settings,
+                                     grad_depth=grad_depth, grad_alpha=grad_alpha, camera=True)
+        g_view = g["viewmatrix"].to(ctx.cam_dtypes[0]) if ctx.needs_input_grad[9] else None
+        g_proj = g["projmatrix"].to(ctx.cam_dtypes[1]) if ctx.needs_input_grad[10] else None
+        return (g["means3D"], g["means2D"], None, g["colors"], g["opacities"], g["scales"], g["rotations"],
+                None, None, g_view, g_proj, None)
+
+
 class GaussianRasterizer(nn.Module):
     def __init__(self, raster_settings: GaussianRasterizationSettings):
         super().__init__()
@@ -421,13 +463,19 @@ class GaussianRasterizer(nn.Module):
         """(color [3,H,W], radii [P]); with depth_alpha=True (color, radii, depth [1,H,W], alpha [1,H,W]):
         depth = sum_i z_i alpha_i T_i, the accumulated view-space depth with background 0, and alpha = 1 - T_final,
         both from the walk that forms the colour and both differentiable.  The expected (normalised) depth is
-        depth / alpha where alpha > 0; the caller forms it."""
+        depth / alpha where alpha > 0; the caller forms it.
+        When the settings' viewmatrix or projmatrix requires grad (and grad mode is on), they receive gradients too."""
         raster_settings = self.raster_settings
         if (shs is None and colors_precomp is None) or (shs is not None and colors_precomp is not None):
             raise Exception('Please provide excatly one of either SHs or precomputed colors!')
         if ((scales is None or rotations is None) and cov3D_precomp is None) or \
                 ((scales is not None or rotations is not None) and cov3D_precomp is not None):
             raise Exception('Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!')
+        if torch.is_grad_enabled() and (raster_settings.viewmatrix.requires_grad or
+                                        raster_settings.projmatrix.requires_grad):
+            return _RasterizeGaussiansCamera.apply(means3D, means2D, shs, colors_precomp, opacities, scales, rotations,
+                                                   cov3D_precomp, raster_settings, raster_settings.viewmatrix,
+                                                   raster_settings.projmatrix, bool(depth_alpha))
         if depth_alpha:
             return _RasterizeGaussiansDepthAlpha.apply(means3D, means2D, shs, colors_precomp, opacities, scales,
                                                        rotations, cov3D_precomp, raster_settings)
