@@ -205,6 +205,38 @@ int splatco_preprocess_bwd_camera(int P, const float *means3D, const float *scal
                                   float *dL_dscales, float *dL_drots, const float *dL_ddepth, void *ws,
                                   float *dL_dview, float *dL_dproj, void *stream);
 
+/* ---- antialiasing (opt-in; the entry points above are unchanged) ------------------------------------
+ * The screen-space mip filter with opacity compensation.  With (a0, b, c0) the projected 2D covariance before the
+ * 0.3 px^2 dilation and (a, b, c) = (a0 + 0.3, b, c0 + 0.3) after it, each Gaussian's opacity is scaled by
+ *     rho = sqrt(max(2.5e-5, (a0 c0 - b^2) / (a c - b^2)))
+ * so that a Gaussian smaller than a pixel keeps its integrated weight instead of being drawn as a full-opacity blob.
+ *
+ * preprocess_fwd_aa / preprocess_fwd_aa_counted: splatco_preprocess_fwd / splatco_preprocess_fwd_counted with the
+ * record's opacity opacities[i] * rho.  radii, tiles, depths, the conic and the rest of the record are bit for bit
+ * those of the plain calls; the binning and blend entry points take the geometry workspace unchanged. */
+int splatco_preprocess_fwd_aa(int P, const float *means3D, const float *scales, int scale_stride,
+                              const float *rots, const float *opacities, const float *colors,
+                              float scale_mod, const float *view, const float *proj, float tanfovx,
+                              float tanfovy, int H, int W, int32_t *radii_out, void *geom,
+                              int32_t *num_rendered_host, void *stream);
+int splatco_preprocess_fwd_aa_counted(int P_max, const int32_t *P_dev, const float *means3D,
+                                      const float *scales, int scale_stride, const float *rots,
+                                      const float *opacities, const float *colors, float scale_mod,
+                                      const float *view, const float *proj, float tanfovx, float tanfovy,
+                                      int H, int W, int32_t *radii_out, void *geom,
+                                      int32_t *num_rendered_host, void *stream);
+/* preprocess_bwd_aa: the preprocess backward of an antialiased forward.  On entry dL_dopacity[P] holds what the blend
+ * backward accumulated (dL / d record opacity); it is rewritten IN PLACE to dL/dopacities = that * rho, and
+ * dL/drho = that * opacities[i] is taken on through (a, b, c) to dL_dmeans3D, dL_dscales and dL_drots.
+ * dL_ddepth [P] may be NULL (as splatco_preprocess_bwd) or given (as splatco_preprocess_bwd_depth).  ws, dL_dview and
+ * dL_dproj are either all NULL or all given (as splatco_preprocess_bwd_camera, including the rho term). */
+int splatco_preprocess_bwd_aa(int P, const float *means3D, const float *scales, int scale_stride,
+                              const float *rots, float scale_mod, const float *view, const float *proj,
+                              float tanfovx, float tanfovy, int H, int W, const int32_t *radii,
+                              const float *dL_dmean2D, const float *dL_dconic, float *dL_dmeans3D,
+                              float *dL_dscales, float *dL_drots, const float *opacities, float *dL_dopacity,
+                              const float *dL_ddepth, void *ws, float *dL_dview, float *dL_dproj, void *stream);
+
 /* ---- anchor decode: replaces generate_neural_gaussians -----------------------------------------
  * (gaussian_renderer/__init__.py:18-116; FeaturePlanes.forward scene/gaussian_model.py:149-169;
  * PlaneGrid scene/grids.py:146-201; heads scene/gaussian_model.py:316-337).

@@ -51,6 +51,9 @@ SIGNATURES = {
     "splatco_preprocess_bwd_depth": (_i, [_i, _vp, _vp, _i, _vp, _f, _vp, _vp, _f, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "splatco_camera_grad_ws_bytes": (_sz, [_i]),
     "splatco_preprocess_bwd_camera": (_i, [_i, _vp, _vp, _i, _vp, _f, _vp, _vp, _f, _f, _i, _i] + [_vp] * 11),
+    "splatco_preprocess_fwd_aa": (_i, [_i, _vp, _vp, _i, _vp, _vp, _vp, _f, _vp, _vp, _f, _f, _i, _i, _vp, _vp, _vp, _vp]),
+    "splatco_preprocess_fwd_aa_counted": (_i, [_i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _f, _vp, _vp, _f, _f, _i, _i, _vp, _vp, _vp, _vp]),
+    "splatco_preprocess_bwd_aa": (_i, [_i, _vp, _vp, _i, _vp, _f, _vp, _vp, _f, _f, _i, _i] + [_vp] * 13),
     # decode: descriptor / gradient structs are passed with ctypes.byref (see decode.py)
     "splatco_pack_planes": (_i, [_i, _i] + [_vp] * 7),
     "splatco_unpack_planes_add": (_i, [_i, _i] + [_vp] * 7),

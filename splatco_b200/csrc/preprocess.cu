@@ -11,6 +11,8 @@
 // Rounding contract: the chain that decides integers (radius, rect, tiles_touched, depth key) uses
 // individually rounded __f*_rn operations in exactly the order of oracle/raster_oracle.c, so the
 // integer outputs are bit-identical to the CPU oracle regardless of nvcc's FMA contraction.
+#include <type_traits>
+
 #include "camgrad.cuh"
 #include "common.cuh"
 
@@ -30,6 +32,7 @@ struct Proj {
     int radius;
     float depth, px, py;
     float conic[3];
+    float rho;                // antialiasing opacity factor (project_one<true> only)
     int r0x, r0y, r1x, r1y;
     uint32_t tiles;
 };
@@ -45,6 +48,9 @@ __device__ __forceinline__ void rect_of(float px, float py, int radius, int gx, 
 }
 
 // view/proj are the 32 floats staged in shared memory by the caller.
+// AA: also o.rho = sqrt(max(2.5e-5, det0 / det)), the ratio of the undilated to the dilated 2D covariance determinant
+// (DESIGN.md §4.5c), on the same pinned-rounding chain as the conic.
+template <bool AA = false>
 __device__ __forceinline__ void project_one(float x, float y, float z, float sx, float sy, float sz,
                                             float4 q, float mod, const float *__restrict__ view,
                                             const float *__restrict__ proj, float tanfovx,
@@ -108,11 +114,13 @@ __device__ __forceinline__ void project_one(float x, float y, float z, float sx,
         B0[l] = DOT3(A0[0], S[0][l], A0[1], S[1][l], A0[2], S[2][l]);
         B1[l] = DOT3(A1[0], S[0][l], A1[1], S[1][l], A1[2], S[2][l]);
     }
-    const float a = ADD(DOT3(B0[0], A0[0], B0[1], A0[1], B0[2], A0[2]), 0.3f);
+    const float a0 = DOT3(B0[0], A0[0], B0[1], A0[1], B0[2], A0[2]);
     const float b = DOT3(B0[0], A1[0], B0[1], A1[1], B0[2], A1[2]);
-    const float c = ADD(DOT3(B1[0], A1[0], B1[1], A1[1], B1[2], A1[2]), 0.3f);
+    const float c0 = DOT3(B1[0], A1[0], B1[1], A1[1], B1[2], A1[2]);
+    const float a = ADD(a0, 0.3f), c = ADD(c0, 0.3f);
     const float det = SUB(MUL(a, c), MUL(b, b));
     if (det == 0.0f) return;
+    if constexpr (AA) o.rho = SQRT(fmaxf(2.5e-5f, DIV(SUB(MUL(a0, c0), MUL(b, b)), det)));
     const float det_inv = DIV(1.0f, det);
     const float mid = MUL(0.5f, ADD(a, c));
     const float sq = SQRT(fmaxf(0.1f, SUB(MUL(mid, mid), det)));
@@ -200,6 +208,8 @@ visible_compact_kernel(int N, const uint8_t *__restrict__ mask, const uint32_t *
 }
 
 // ---- preprocess forward: also emits per-block tile-count sums (first level of the scan) ---------
+// AA: the record's opacity is opacities[i] * rho (project_one<true>); everything else is that of the plain kernel.
+template <bool AA>
 __global__ void __launch_bounds__(PRE_THREADS)
 preprocess_fwd_kernel(int P, const uint32_t *__restrict__ P_dev, const float *__restrict__ means3D, const float *__restrict__ scales,
                       int scale_stride, const float *__restrict__ rots,
@@ -223,14 +233,14 @@ preprocess_fwd_kernel(int P, const uint32_t *__restrict__ P_dev, const float *__
         const float *sp = scales + (size_t)scale_stride * i;
         const float4 q = *reinterpret_cast<const float4 *>(rots + 4 * (size_t)i);
         Proj o;
-        project_one(x, y, z, sp[0], sp[1], sp[2], q, mod, s_cam, s_cam + 16, tanfovx, tanfovy, fx, fy, H, W, gx, gy, o);
+        project_one<AA>(x, y, z, sp[0], sp[1], sp[2], q, mod, s_cam, s_cam + 16, tanfovx, tanfovy, fx, fy, H, W, gx, gy, o);
         radii[i] = o.radius;
         tiles[i] = o.tiles;
         depths[i] = o.depth;
         t = o.tiles;
         float4 r0, r1, r2;
         if (o.radius > 0) {
-            const float op = opacities[i];
+            const float op = AA ? MUL(opacities[i], o.rho) : opacities[i];
             const float cr = colors[3 * (size_t)i], cg = colors[3 * (size_t)i + 1], cb = colors[3 * (size_t)i + 2];
             r0 = make_float4(o.px, o.py, o.conic[0], o.conic[1]);
             r1 = make_float4(o.conic[2], op, cr, cg);
@@ -255,10 +265,42 @@ preprocess_fwd_kernel(int P, const uint32_t *__restrict__ P_dev, const float *__
 }
 
 // ---- per-Gaussian backward chain (fp32; tolerance-compared, so the compiler may contract) --------
-// DEPTH: the blend's dL/dz_view (the one trailing argument, `const float *dL_ddepth`) is added to dL/dmeans3D through
-// dz_view/dmean = (V[2], V[6], V[10]).  It is a parameter pack, empty without DEPTH, so that preprocess_bwd_kernel<false>
-// keeps the parameter list -- and with it the code -- of the colour-only kernel.
+// DEPTH: the blend's dL/dz_view (the trailing argument `const float *dL_ddepth`) is added to dL/dmeans3D through
+// dz_view/dmean = (V[2], V[6], V[10]).
+// Antialiasing: a trailing AAOpacity (after dL_ddepth when DEPTH) adds the opacity factor rho's term to dL/d(a, b, c)
+// and rewrites dL_dopacity in place from dL/d(record opacity) to dL/dopacities (aa_rho_grad).
+// The trailing arguments are a parameter pack, empty for the colour-only call, so that preprocess_bwd_kernel<false> keeps
+// the parameter list -- and with it the code -- of the colour-only kernel.
+struct AAOpacity {
+    const float *opacities;
+    float *dL_dopacity;
+};
 __device__ __forceinline__ const float *depth_grad_ptr(const float *p) { return p; }
+__device__ __forceinline__ const float *depth_grad_ptr(const float *p, AAOpacity) { return p; }
+__device__ __forceinline__ AAOpacity aa_args(AAOpacity a) { return a; }
+__device__ __forceinline__ AAOpacity aa_args(const float *, AAOpacity a) { return a; }
+template <typename... T> constexpr bool has_aa = (std::is_same<T, AAOpacity>::value || ... || false);
+
+// rho = sqrt(max(2.5e-5, det0 / det)) with det0 = a0 c0 - b^2 of the undilated and det = a c - b^2 of the dilated
+// (a = a0 + 0.3, c = c0 + 0.3) 2D covariance.  Where the clamp is inactive, adds dL/drho * drho/d(a, b, c) to
+// (dL_da, dL_db, dL_dc), with the exact derivatives in cancellation-free form:
+//     drho/da = (c0 det - det0 c) / (2 rho det^2) = 0.3 (c c0 + b^2) / (2 rho det^2)
+//     drho/dc = (a0 det - det0 a) / (2 rho det^2) = 0.3 (a a0 + b^2) / (2 rho det^2)
+//     drho/db = b (det0 - det) / (rho det^2)       = -0.3 b (a + c0) / (rho det^2)
+// Returns rho.
+__device__ __forceinline__ float aa_rho_grad(float a0, float b, float c0, float a, float c, float det, float dL_drho,
+                                             float &dL_da, float &dL_db, float &dL_dc) {
+    const float ratio = (a0 * c0 - b * b) / det;
+    if (!(ratio > 2.5e-5f)) return sqrtf(2.5e-5f);
+    const float rho = sqrtf(ratio);
+    const float idet = 1.f / det;
+    const float k = 0.15f * dL_drho / rho * idet * idet;        // 0.3 dL/drho / (2 rho det^2)
+    dL_da += k * (c * c0 + b * b);
+    dL_dc += k * (a * a0 + b * b);
+    dL_db -= 2.f * k * b * (a + c0);
+    return rho;
+}
+
 template <bool DEPTH, typename... DepthGrad>
 __global__ void __launch_bounds__(PRE_THREADS)
 preprocess_bwd_kernel(int P, const float *__restrict__ means3D, const float *__restrict__ scales,
@@ -320,9 +362,17 @@ preprocess_bwd_kernel(int P, const float *__restrict__ means3D, const float *__r
         const float denom = a * c - b * b;
         const float d2inv = 1.0f / (denom * denom + 0.0000001f);   // reference quirk (SURVEY A.5)
         const float gc0 = dL_dconic[3 * (size_t)i], gc1 = dL_dconic[3 * (size_t)i + 1], gc2 = dL_dconic[3 * (size_t)i + 2];
-        const float dL_da = d2inv * (-c * c * gc0 + 2.f * b * c * gc1 + (denom - a * c) * gc2);
-        const float dL_dc = d2inv * (-a * a * gc2 + 2.f * a * b * gc1 + (denom - a * c) * gc0);
-        const float dL_db = d2inv * 2.f * (b * c * gc0 - (denom + 2.f * b * b) * gc1 + a * b * gc2);
+        float dL_da = d2inv * (-c * c * gc0 + 2.f * b * c * gc1 + (denom - a * c) * gc2);
+        float dL_dc = d2inv * (-a * a * gc2 + 2.f * a * b * gc1 + (denom - a * c) * gc0);
+        float dL_db = d2inv * 2.f * (b * c * gc0 - (denom + 2.f * b * b) * gc1 + a * b * gc2);
+        if constexpr (has_aa<DepthGrad...>) {
+            const AAOpacity aa = aa_args(dL_ddepth...);
+            const float a0 = B[0][0] * A[0][0] + B[0][1] * A[0][1] + B[0][2] * A[0][2];
+            const float c0 = B[1][0] * A[1][0] + B[1][1] * A[1][1] + B[1][2] * A[1][2];
+            const float g = aa.dL_dopacity[i];
+            const float rho = aa_rho_grad(a0, b, c0, a, c, denom, g * aa.opacities[i], dL_da, dL_db, dL_dc);
+            aa.dL_dopacity[i] = g * rho;
+        }
         const float G2[2][2] = { { dL_da, 0.5f * dL_db }, { 0.5f * dL_db, dL_dc } };
         // GA = G2 A (2x3);  dS = A^T GA;  dA = 2 G2 B
         float GA[2][3], dS[3][3], dA[2][3];
@@ -393,13 +443,16 @@ preprocess_bwd_kernel(int P, const float *__restrict__ means3D, const float *__r
 //     dV[4k]    += dA[0][k] J00,   dV[4k+1] += dA[1][k] J11,   dV[4k+2] += dA[0][k] J02 + dA[1][k] J12   (k < 3)
 //     dPm[4k]   += g2x mw p~_k,    dPm[4k+1] += g2y mw p~_k,   dPm[4k+3] += -(g2x hx + g2y hy) mw^2 p~_k
 // into part[blockIdx.x][0..31] (camgrad.cuh).  The forward never reads V[3,7,11,15] or Pm[2,6,10,14]: those stay 0.
+// Antialiasing: a trailing AAOpacity adds the rho term to dL/d(a, b, c) as preprocess_bwd_kernel does.  This kernel only
+// reads dL_dopacity, which must still hold dL/d(record opacity): it runs before the per-Gaussian kernel rewrites it.
+template <typename... AA>
 __global__ void __launch_bounds__(PRE_THREADS)
 preprocess_bwd_camera_kernel(int P, const float *__restrict__ means3D, const float *__restrict__ scales,
                              int scale_stride, const float *__restrict__ rots, float mod,
                              const float *__restrict__ view, const float *__restrict__ proj, float tanfovx,
                              float tanfovy, float fx, float fy, const int32_t *__restrict__ radii,
                              const float *__restrict__ dL_dmean2D, const float *__restrict__ dL_dconic,
-                             const float *__restrict__ dL_ddepth, float *__restrict__ part) {
+                             const float *__restrict__ dL_ddepth, float *__restrict__ part, AA... aa_opacity) {
     static_assert(PRE_THREADS == CAM_ROWS, "one camera partial per preprocess CTA");
     __shared__ float s_cam[32];
     stage_cam(s_cam, view, proj);
@@ -452,9 +505,15 @@ preprocess_bwd_camera_kernel(int P, const float *__restrict__ means3D, const flo
         const float denom = a * c - b * b;
         const float d2inv = 1.0f / (denom * denom + 0.0000001f);
         const float gc0 = dL_dconic[3 * (size_t)i], gc1 = dL_dconic[3 * (size_t)i + 1], gc2 = dL_dconic[3 * (size_t)i + 2];
-        const float dL_da = d2inv * (-c * c * gc0 + 2.f * b * c * gc1 + (denom - a * c) * gc2);
-        const float dL_dc = d2inv * (-a * a * gc2 + 2.f * a * b * gc1 + (denom - a * c) * gc0);
-        const float dL_db = d2inv * 2.f * (b * c * gc0 - (denom + 2.f * b * b) * gc1 + a * b * gc2);
+        float dL_da = d2inv * (-c * c * gc0 + 2.f * b * c * gc1 + (denom - a * c) * gc2);
+        float dL_dc = d2inv * (-a * a * gc2 + 2.f * a * b * gc1 + (denom - a * c) * gc0);
+        float dL_db = d2inv * 2.f * (b * c * gc0 - (denom + 2.f * b * b) * gc1 + a * b * gc2);
+        if constexpr (sizeof...(AA) > 0) {
+            const AAOpacity aa = aa_args(aa_opacity...);
+            const float a0 = B[0][0] * A[0][0] + B[0][1] * A[0][1] + B[0][2] * A[0][2];
+            const float c0 = B[1][0] * A[1][0] + B[1][1] * A[1][1] + B[1][2] * A[1][2];
+            aa_rho_grad(a0, b, c0, a, c, denom, aa.dL_dopacity[i] * aa.opacities[i], dL_da, dL_db, dL_dc);
+        }
         const float G2[2][2] = { { dL_da, 0.5f * dL_db }, { 0.5f * dL_db, dL_dc } };
         float dA[2][3];
 #pragma unroll
@@ -552,6 +611,7 @@ extern "C" int splatco_visible_filter_compact(int N, const float *means3D, const
     return 0;
 }
 
+template <bool AA>
 static int preprocess_fwd_impl(int P, const uint32_t *P_dev, const float *means3D, const float *scales, int scale_stride,
                                const float *rots, const float *opacities, const float *colors,
                                float scale_mod, const float *view, const float *proj,
@@ -572,9 +632,9 @@ static int preprocess_fwd_impl(int P, const uint32_t *P_dev, const float *means3
     const float fx = (float)W / (2.0f * tanfovx), fy = (float)H / (2.0f * tanfovy);
     const int gx = ceil_div(W, TILE), gy = ceil_div(H, TILE);
     const int nb = ceil_div(P, PRE_THREADS);
-    preprocess_fwd_kernel<<<nb, PRE_THREADS, 0, st>>>(P, P_dev, means3D, scales, scale_stride, rots, opacities, colors,
-                                                      scale_mod, view, proj, tanfovx, tanfovy, fx, fy, H, W,
-                                                      gx, gy, radii_out, g.rec, g.depths, g.tiles, g.block_sums);
+    preprocess_fwd_kernel<AA><<<nb, PRE_THREADS, 0, st>>>(P, P_dev, means3D, scales, scale_stride, rots, opacities, colors,
+                                                          scale_mod, view, proj, tanfovx, tanfovy, fx, fy, H, W,
+                                                          gx, gy, radii_out, g.rec, g.depths, g.tiles, g.block_sums);
     SPLATCO_CHECK_LAUNCH();
     scan_block_sums_kernel<<<1, 1024, 0, st>>>(nb, g.block_sums, g.block_offsets, g.total);
     SPLATCO_CHECK_LAUNCH();
@@ -588,7 +648,7 @@ extern "C" int splatco_preprocess_fwd(int P, const float *means3D, const float *
                                       float scale_mod, const float *view, const float *proj,
                                       float tanfovx, float tanfovy, int H, int W, int32_t *radii_out,
                                       void *geom, int32_t *num_rendered_host, void *stream) {
-    return preprocess_fwd_impl(P, nullptr, means3D, scales, scale_stride, rots, opacities, colors, scale_mod, view, proj,
+    return preprocess_fwd_impl<false>(P, nullptr, means3D, scales, scale_stride, rots, opacities, colors, scale_mod, view, proj,
                                tanfovx, tanfovy, H, W, radii_out, geom, num_rendered_host, stream);
 }
 
@@ -599,17 +659,39 @@ extern "C" int splatco_preprocess_fwd_counted(int P_max, const int32_t *P_dev, c
                                               float tanfovy, int H, int W, int32_t *radii_out, void *geom,
                                               int32_t *num_rendered_host, void *stream) {
     SPLATCO_REQUIRE(P_dev, "preprocess_fwd_counted: null device count");
-    return preprocess_fwd_impl(P_max, reinterpret_cast<const uint32_t *>(P_dev), means3D, scales, scale_stride, rots,
+    return preprocess_fwd_impl<false>(P_max, reinterpret_cast<const uint32_t *>(P_dev), means3D, scales, scale_stride, rots,
                                opacities, colors, scale_mod, view, proj, tanfovx, tanfovy, H, W, radii_out, geom,
                                num_rendered_host, stream);
 }
 
-template <bool DEPTH>
+extern "C" int splatco_preprocess_fwd_aa(int P, const float *means3D, const float *scales, int scale_stride,
+                                         const float *rots, const float *opacities, const float *colors,
+                                         float scale_mod, const float *view, const float *proj,
+                                         float tanfovx, float tanfovy, int H, int W, int32_t *radii_out,
+                                         void *geom, int32_t *num_rendered_host, void *stream) {
+    return preprocess_fwd_impl<true>(P, nullptr, means3D, scales, scale_stride, rots, opacities, colors, scale_mod, view,
+                                     proj, tanfovx, tanfovy, H, W, radii_out, geom, num_rendered_host, stream);
+}
+
+extern "C" int splatco_preprocess_fwd_aa_counted(int P_max, const int32_t *P_dev, const float *means3D,
+                                                 const float *scales, int scale_stride, const float *rots,
+                                                 const float *opacities, const float *colors, float scale_mod,
+                                                 const float *view, const float *proj, float tanfovx,
+                                                 float tanfovy, int H, int W, int32_t *radii_out, void *geom,
+                                                 int32_t *num_rendered_host, void *stream) {
+    SPLATCO_REQUIRE(P_dev, "preprocess_fwd_aa_counted: null device count");
+    return preprocess_fwd_impl<true>(P_max, reinterpret_cast<const uint32_t *>(P_dev), means3D, scales, scale_stride,
+                                     rots, opacities, colors, scale_mod, view, proj, tanfovx, tanfovy, H, W, radii_out,
+                                     geom, num_rendered_host, stream);
+}
+
+// AA: empty, or one AAOpacity (the antialiased backward), passed on to preprocess_bwd_kernel
+template <bool DEPTH, typename... AA>
 static int preprocess_bwd_impl(const char *name, int P, const float *means3D, const float *scales, int scale_stride,
                                const float *rots, float scale_mod, const float *view, const float *proj, float tanfovx,
                                float tanfovy, int H, int W, const int32_t *radii, const float *dL_dmean2D,
                                const float *dL_dconic, float *dL_dmeans3D, float *dL_dscales, float *dL_drots,
-                               const float *dL_ddepth, void *stream) {
+                               const float *dL_ddepth, void *stream, AA... aa) {
     SPLATCO_REQUIRE(P >= 0 && H > 0 && W > 0, "%s: bad sizes", name);
     if (P == 0) return 0;
     SPLATCO_REQUIRE(means3D && scales && rots && view && proj && radii && dL_dmean2D && dL_dconic &&
@@ -618,13 +700,13 @@ static int preprocess_bwd_impl(const char *name, int P, const float *means3D, co
                     "%s: rotations / dL_drots must be 16-byte aligned", name);
     const float fx = (float)W / (2.0f * tanfovx), fy = (float)H / (2.0f * tanfovy);
     if constexpr (DEPTH)
-        preprocess_bwd_kernel<true, const float *><<<ceil_div(P, PRE_THREADS), PRE_THREADS, 0, (cudaStream_t)stream>>>(
+        preprocess_bwd_kernel<true, const float *, AA...><<<ceil_div(P, PRE_THREADS), PRE_THREADS, 0, (cudaStream_t)stream>>>(
             P, means3D, scales, scale_stride, rots, scale_mod, view, proj, tanfovx, tanfovy, fx, fy, radii,
-            dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales, dL_drots, dL_ddepth);
+            dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales, dL_drots, dL_ddepth, aa...);
     else
-        preprocess_bwd_kernel<false><<<ceil_div(P, PRE_THREADS), PRE_THREADS, 0, (cudaStream_t)stream>>>(
+        preprocess_bwd_kernel<false, AA...><<<ceil_div(P, PRE_THREADS), PRE_THREADS, 0, (cudaStream_t)stream>>>(
             P, means3D, scales, scale_stride, rots, scale_mod, view, proj, tanfovx, tanfovy, fx, fy, radii,
-            dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales, dL_drots);
+            dL_dmean2D, dL_dconic, dL_dmeans3D, dL_dscales, dL_drots, aa...);
     SPLATCO_CHECK_LAUNCH();
     return 0;
 }
@@ -679,11 +761,56 @@ extern "C" int splatco_preprocess_bwd_camera(int P, const float *means3D, const 
     const float fx = (float)W / (2.0f * tanfovx), fy = (float)H / (2.0f * tanfovy);
     const int nb = ceil_div(P, PRE_THREADS);
     float *part = (float *)ws;
-    preprocess_bwd_camera_kernel<<<nb, PRE_THREADS, 0, st>>>(P, means3D, scales, scale_stride, rots, scale_mod, view, proj,
+    preprocess_bwd_camera_kernel<><<<nb, PRE_THREADS, 0, st>>>(P, means3D, scales, scale_stride, rots, scale_mod, view, proj,
                                                              tanfovx, tanfovy, fx, fy, radii, dL_dmean2D, dL_dconic,
                                                              dL_ddepth, part);
     SPLATCO_CHECK_LAUNCH();
     camera_sum_kernel<<<1, 1024, 0, st>>>(nb, 32, 16, 1.0f, part, dL_dview, dL_dproj);
     SPLATCO_CHECK_LAUNCH();
     return 0;
+}
+
+extern "C" int splatco_preprocess_bwd_aa(int P, const float *means3D, const float *scales, int scale_stride,
+                                         const float *rots, float scale_mod, const float *view,
+                                         const float *proj, float tanfovx, float tanfovy, int H, int W,
+                                         const int32_t *radii, const float *dL_dmean2D,
+                                         const float *dL_dconic, float *dL_dmeans3D, float *dL_dscales,
+                                         float *dL_drots, const float *opacities, float *dL_dopacity,
+                                         const float *dL_ddepth, void *ws, float *dL_dview, float *dL_dproj,
+                                         void *stream) {
+    SPLATCO_REQUIRE(P >= 0 && H > 0 && W > 0, "preprocess_bwd_aa: bad sizes");
+    const bool camera = dL_dview || dL_dproj;
+    SPLATCO_REQUIRE(!camera || (dL_dview && dL_dproj && (P == 0 || ws)), "preprocess_bwd_aa: camera outputs need "
+                    "dL_dview, dL_dproj and ws together");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (P == 0) {
+        if (camera) {
+            SPLATCO_CHECK_CUDA(cudaMemsetAsync(dL_dview, 0, 16 * sizeof(float), st));
+            SPLATCO_CHECK_CUDA(cudaMemsetAsync(dL_dproj, 0, 16 * sizeof(float), st));
+        }
+        return 0;
+    }
+    SPLATCO_REQUIRE(opacities && dL_dopacity, "preprocess_bwd_aa: null pointer");
+    const AAOpacity aa{opacities, dL_dopacity};
+    if (camera) {
+        // before the per-Gaussian kernel: it reads dL_dopacity as the blend wrote it
+        SPLATCO_REQUIRE(means3D && scales && rots && view && proj && radii && dL_dmean2D && dL_dconic,
+                        "preprocess_bwd_aa: null pointer");
+        SPLATCO_REQUIRE(((uintptr_t)rots & 15) == 0, "preprocess_bwd_aa: rotations must be 16-byte aligned");
+        const float fx = (float)W / (2.0f * tanfovx), fy = (float)H / (2.0f * tanfovy);
+        const int nb = ceil_div(P, PRE_THREADS);
+        float *part = (float *)ws;
+        preprocess_bwd_camera_kernel<AAOpacity><<<nb, PRE_THREADS, 0, st>>>(
+            P, means3D, scales, scale_stride, rots, scale_mod, view, proj, tanfovx, tanfovy, fx, fy, radii, dL_dmean2D,
+            dL_dconic, dL_ddepth, part, aa);
+        SPLATCO_CHECK_LAUNCH();
+        camera_sum_kernel<<<1, 1024, 0, st>>>(nb, 32, 16, 1.0f, part, dL_dview, dL_dproj);
+        SPLATCO_CHECK_LAUNCH();
+    }
+    return dL_ddepth ? preprocess_bwd_impl<true>("preprocess_bwd_aa", P, means3D, scales, scale_stride, rots, scale_mod,
+                                                 view, proj, tanfovx, tanfovy, H, W, radii, dL_dmean2D, dL_dconic,
+                                                 dL_dmeans3D, dL_dscales, dL_drots, dL_ddepth, stream, aa)
+                     : preprocess_bwd_impl<false>("preprocess_bwd_aa", P, means3D, scales, scale_stride, rots, scale_mod,
+                                                  view, proj, tanfovx, tanfovy, H, W, radii, dL_dmean2D, dL_dconic,
+                                                  dL_dmeans3D, dL_dscales, dL_drots, nullptr, stream, aa);
 }

@@ -38,6 +38,9 @@ class GaussianRasterizationSettings(NamedTuple):
     campos: torch.Tensor
     prefiltered: bool
     debug: bool
+    # screen-space mip filter with opacity compensation (upstream's `antialiasing`): each Gaussian's opacity is scaled
+    # by rho = sqrt(max(2.5e-5, det(cov2D) / det(cov2D + 0.3 I))), so sub-pixel Gaussians keep their integrated weight
+    antialiasing: bool = False
 
 
 _tls = threading.local()
@@ -120,12 +123,12 @@ def preprocess_speculative(xyz_b, color_b, opacity_b, scaling_b, rot_b, count_pt
     sp.geom = _lib.empty_u8(L.splatco_geom_bytes(PL), dev)
     sp.counter = _pinned_counter(dev, 1)
     view, proj = _f32c(settings.viewmatrix), _f32c(settings.projmatrix)
+    name = "splatco_preprocess_fwd_aa_counted" if settings.antialiasing else "splatco_preprocess_fwd_counted"
     with stage("preprocess_fwd"):
-        check(L.splatco_preprocess_fwd_counted(PL, count_ptr, ptr(xyz_b), ptr(scaling_b), 3, ptr(rot_b), ptr(opacity_b),
-                                               ptr(color_b), float(settings.scale_modifier), ptr(view), ptr(proj),
-                                               float(settings.tanfovx), float(settings.tanfovy), H, W,
-                                               ptr(sp.radii_full), ptr(sp.geom), sp.counter.data_ptr(),
-                                               _stream_ptr(dev)), "splatco_preprocess_fwd_counted")
+        check(getattr(L, name)(PL, count_ptr, ptr(xyz_b), ptr(scaling_b), 3, ptr(rot_b), ptr(opacity_b), ptr(color_b),
+                               float(settings.scale_modifier), ptr(view), ptr(proj), float(settings.tanfovx),
+                               float(settings.tanfovy), H, W, ptr(sp.radii_full), ptr(sp.geom), sp.counter.data_ptr(),
+                               _stream_ptr(dev)), name)
     # M and R are complete once this event has passed; the caller waits for IT, not for the stream
     sp.event = torch.cuda.Event()
     sp.event.record(torch.cuda.current_stream(dev))
@@ -251,11 +254,12 @@ def rasterize_forward_state(means3D, colors, opacities, scales, rotations, setti
             radii = radii_full = _lib.empty_rows(P, None, torch.int32, dev)
             geom = _lib.empty_u8(L.splatco_geom_bytes(P), dev)
             counter = _pinned_counter(dev)
+            name = "splatco_preprocess_fwd_aa" if settings.antialiasing else "splatco_preprocess_fwd"
             with stage("preprocess_fwd"):
-                check(L.splatco_preprocess_fwd(P, ptr(means3D), ptr(scales), sstride, ptr(rotations), ptr(opacities),
-                                               ptr(colors), float(settings.scale_modifier), ptr(view), ptr(proj),
-                                               float(settings.tanfovx), float(settings.tanfovy), H, W, ptr(radii),
-                                               ptr(geom), counter.data_ptr(), stream), "splatco_preprocess_fwd")
+                check(getattr(L, name)(P, ptr(means3D), ptr(scales), sstride, ptr(rotations), ptr(opacities), ptr(colors),
+                                       float(settings.scale_modifier), ptr(view), ptr(proj), float(settings.tanfovx),
+                                       float(settings.tanfovy), H, W, ptr(radii), ptr(geom), counter.data_ptr(), stream),
+                      name)
             # the one device->host sync of the forward (the reference has the same one, SURVEY §3.1)
             torch.cuda.current_stream(dev).synchronize()
             R = int(counter[0])
@@ -282,15 +286,20 @@ def rasterize_forward_state(means3D, colors, opacities, scales, rotations, setti
 
 
 def rasterize_backward_state(st: RasterState, grad_color, means3D, scales, rotations, settings, grad_depth=None,
-                             grad_alpha=None, camera=False):
+                             grad_alpha=None, camera=False, opacities=None):
     """Backward pass; returns dict of gradients (all fp32, same row count as the inputs).
     grad_depth / grad_alpha ([1,H,W] or None) need a depth_alpha forward.  With both None this is the colour-only
     backward (splatco_blend_bwd + splatco_preprocess_bwd); with either given, splatco_blend_bwd_depth_alpha also
     yields dL/dz_view per Gaussian (returned as "depth"), which splatco_preprocess_bwd_depth adds to dL/dmeans3D, and
     grad_color may be None.  Absent upstream gradients are passed as NULL (zero).
     camera=True: splatco_preprocess_bwd_camera replaces the preprocess backward (same per-Gaussian outputs) and the dict
-    also holds "viewmatrix" and "projmatrix", fp32 [4,4]: the gradients of the contiguous fp32 copies the kernels read."""
+    also holds "viewmatrix" and "projmatrix", fp32 [4,4]: the gradients of the contiguous fp32 copies the kernels read.
+    settings.antialiasing: splatco_preprocess_bwd_aa serves all of the above; it needs the forward's `opacities` and turns
+    the blend's gradient with respect to the record's compensated opacity into dL/dopacities."""
     da = grad_depth is not None or grad_alpha is not None
+    aa = bool(settings.antialiasing)
+    if aa and opacities is None:
+        raise RuntimeError("an antialiased backward needs the forward's opacities")
     if da and not st.depth_alpha:
         raise RuntimeError("depth / alpha gradients need a forward with depth_alpha=True")
     L = _lib.lib()
@@ -337,7 +346,13 @@ def rasterize_backward_state(st: RasterState, grad_color, means3D, scales, rotat
                 check(L.splatco_blend_bwd(P, R, H, W, *ws, ptr(grad_color), *blend_out, stream), "splatco_blend_bwd")
         _debug_sync(settings, "blend_bwd")
         with stage("preprocess_bwd"):
-            if camera:
+            if aa:
+                opacities = _f32c(opacities)
+                cam_ws = _lib.empty_u8(L.splatco_camera_grad_ws_bytes(P), dev) if camera else None
+                cam = (ptr(cam_ws), ptr(out["viewmatrix"]), ptr(out["projmatrix"])) if camera else (None, None, None)
+                check(L.splatco_preprocess_bwd_aa(*pre_args, ptr(opacities), ptr(g_opac), ptr(g_depth), *cam, stream),
+                      "splatco_preprocess_bwd_aa")
+            elif camera:
                 cam_ws = _lib.empty_u8(L.splatco_camera_grad_ws_bytes(P), dev)
                 check(L.splatco_preprocess_bwd_camera(*pre_args, ptr(g_depth), ptr(cam_ws), ptr(out["viewmatrix"]),
                                                       ptr(out["projmatrix"]), stream), "splatco_preprocess_bwd_camera")
@@ -356,12 +371,19 @@ def _check_supported(sh, cov3Ds_precomp):
         raise NotImplementedError("splatco_b200: cov3D_precomp is not on SplatCo's path (it passes scales+rotations)")
 
 
-def _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations):
+def _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations, opacities):
     ctx.raster_settings = raster_settings
     ctx.state = st
-    ctx.save_for_backward(means3D, scales, rotations)
+    # the antialiased backward also reads the opacities (dL/dopacities = rho dL/d(record opacity))
+    ctx.save_for_backward(means3D, scales, rotations, *((opacities,) if raster_settings.antialiasing else ()))
     ctx.mark_non_differentiable(radii)
     ctx.set_materialize_grads(False)          # no zero-filled gradient tensor for `radii` (or an unused map)
+
+
+def _saved(ctx):
+    """(means3D, scales, rotations, opacities or None)"""
+    t = ctx.saved_tensors
+    return (*t, None) if len(t) == 3 else t
 
 
 class _RasterizeGaussians(torch.autograd.Function):
@@ -371,15 +393,16 @@ class _RasterizeGaussians(torch.autograd.Function):
         _check_supported(sh, cov3Ds_precomp)
         color, radii, st = rasterize_forward_state(means3D, colors_precomp, opacities, scales, rotations,
                                                    raster_settings)
-        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations)
+        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations, opacities)
         return color, radii
 
     @staticmethod
     def backward(ctx, grad_out_color, _grad_radii):
         if grad_out_color is None:
             return (None,) * 9
-        means3D, scales, rotations = ctx.saved_tensors
-        g = rasterize_backward_state(ctx.state, grad_out_color, means3D, scales, rotations, ctx.raster_settings)
+        means3D, scales, rotations, opacities = _saved(ctx)
+        g = rasterize_backward_state(ctx.state, grad_out_color, means3D, scales, rotations, ctx.raster_settings,
+                                     opacities=opacities)
         # (means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, settings)
         return (g["means3D"], g["means2D"], None, g["colors"], g["opacities"], g["scales"], g["rotations"],
                 None, None)
@@ -402,17 +425,17 @@ class _RasterizeGaussiansDepthAlpha(torch.autograd.Function):
                                                    raster_settings, depth_alpha=True)
         depth, alpha = st.depth, st.alpha
         st.depth = st.alpha = None                  # the state outlives the outputs in ctx; it does not need them
-        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations)
+        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations, opacities)
         return color, radii, depth, alpha
 
     @staticmethod
     def backward(ctx, grad_out_color, _grad_radii, grad_depth, grad_alpha):
         if grad_out_color is None and grad_depth is None and grad_alpha is None:
             return (None,) * 9
-        means3D, scales, rotations = ctx.saved_tensors
+        means3D, scales, rotations, opacities = _saved(ctx)
         # both map gradients None: exactly the colour-only backward (splatco_blend_bwd + splatco_preprocess_bwd)
         g = rasterize_backward_state(ctx.state, grad_out_color, means3D, scales, rotations, ctx.raster_settings,
-                                     grad_depth=grad_depth, grad_alpha=grad_alpha)
+                                     grad_depth=grad_depth, grad_alpha=grad_alpha, opacities=opacities)
         return (g["means3D"], g["means2D"], None, g["colors"], g["opacities"], g["scales"], g["rotations"],
                 None, None)
 
@@ -429,7 +452,7 @@ class _RasterizeGaussiansCamera(torch.autograd.Function):
         _check_supported(sh, cov3Ds_precomp)
         color, radii, st = rasterize_forward_state(means3D, colors_precomp, opacities, scales, rotations,
                                                    raster_settings, depth_alpha=depth_alpha)
-        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations)
+        _save_for_backward(ctx, st, raster_settings, radii, means3D, scales, rotations, opacities)
         ctx.cam_dtypes = (viewmatrix.dtype, projmatrix.dtype)
         if not depth_alpha:
             return color, radii
@@ -441,9 +464,9 @@ class _RasterizeGaussiansCamera(torch.autograd.Function):
     def backward(ctx, grad_out_color, _grad_radii, grad_depth=None, grad_alpha=None):
         if grad_out_color is None and grad_depth is None and grad_alpha is None:
             return (None,) * 12
-        means3D, scales, rotations = ctx.saved_tensors
+        means3D, scales, rotations, opacities = _saved(ctx)
         g = rasterize_backward_state(ctx.state, grad_out_color, means3D, scales, rotations, ctx.raster_settings,
-                                     grad_depth=grad_depth, grad_alpha=grad_alpha, camera=True)
+                                     grad_depth=grad_depth, grad_alpha=grad_alpha, camera=True, opacities=opacities)
         g_view = g["viewmatrix"].to(ctx.cam_dtypes[0]) if ctx.needs_input_grad[9] else None
         g_proj = g["projmatrix"].to(ctx.cam_dtypes[1]) if ctx.needs_input_grad[10] else None
         return (g["means3D"], g["means2D"], None, g["colors"], g["opacities"], g["scales"], g["rotations"],

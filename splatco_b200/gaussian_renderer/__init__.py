@@ -44,6 +44,7 @@ def _settings(viewpoint_camera, pipe, bg_color, scaling_modifier):
         campos=viewpoint_camera.camera_center,
         prefiltered=False,
         debug=pipe.debug,
+        antialiasing=bool(getattr(pipe, "antialiasing", False)),   # upstream PipelineParams' flag; off when absent
     )
 
 
